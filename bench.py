@@ -9,6 +9,8 @@ A "step" is one UCT_search (`--sims` simulations per tree, default 800) for ever
 root positions, with Dirichlet root noise (0.8, 0.25) and the reference's SimpleNN (random-init,
 seed 0) as leaf evaluator.  One process per GPU; games are sharded by index, there is no data-path
 collective (weak scaling).  Rank 0 prints ONE JSON line (stdout carries nothing else).
+`--dump-outputs DIR` also writes what the last timed step computed as .npy files; the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 
 The engine's eval cache (the reference's LRU of net outputs, utils/proxies.py:23-26) is part of the path and is
 EMPTIED at the start of every step, inside the timed region.  Keys of the line beyond the contract:
@@ -85,7 +87,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-workers", type=int, default=0, help="processes for the CPU baseline (0 = min(cores-1, 64))")
     ap.add_argument("--cpu-positions", type=int, default=2, help="searches per worker in the bounded CPU sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (root visits, W and priors of every game; the end-to-end "
+                         "arm's visits) to DIR/<name>.npy, float32/float64, at most 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def workload_name(args):
@@ -260,6 +270,20 @@ def host_noise(rs, valid_np, alpha):
     import numpy as np
     A = valid_np.shape[1]
     return rs.dirichlet(np.ones(A) * alpha, size=valid_np.shape[0]) * valid_np  # mcts.py:220-223
+
+
+def dump_outputs(path, arrays, limit=64 << 20):
+    """Writes every array as path/<name>.npy.  The arrays share their first axis (the game); when they exceed `limit`
+    bytes in all, a fixed seeded sample of games is written instead, the same one in every run with the same arguments."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    total = sum(a.nbytes for a in arrays.values())
+    rows = np.arange(n)
+    if total > limit:
+        rows = np.sort(np.random.RandomState(0).choice(n, n * limit // total, replace=False))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a[rows])
 
 
 def sub_bench(extra, timeout=420):
@@ -567,10 +591,18 @@ def main():
     launches = eng.n_launches - l0
     waves_per_step = (eng.n_waves - w0) / args.steps
     st = eng.status()  # also checks that no tree faulted
+    outputs = None
+    if args.dump_outputs:  # the trees of the last timed step, read before anything else runs on the engine
+        W, P, _, _ = eng.root_children()
+        outputs = {"root_visits": visits.float().cpu().numpy(), "root_W": W.cpu().numpy(), "root_priors": P.cpu().numpy()}
     for _ in range(2):
         step_e2e()
     ms_e2e, wall_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:
+        outputs["e2e_root_visits"] = visits_host.float().numpy()
+        dump_outputs(args.dump_outputs, {(k if world == 1 else "%s_rank%d" % (k, rank)): v for k, v in outputs.items()},
+                     limit=(64 << 20) // world)
 
     sims_per_step = args.games * args.sims * world
     value = sims_per_step * args.steps / (ms / 1e3)
