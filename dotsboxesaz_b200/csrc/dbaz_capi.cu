@@ -444,6 +444,7 @@ int dbaz_nn_heads(dbaz_engine* e, const void* logits, int32_t ld, int32_t dtype,
                   uint64_t stream) {
     if (!e || !logits || !priors || !values) return 1;
     if (n <= 0) return 0;
+    if (ld < e->board.A + 1) return fail(e, "dbaz_nn_heads: ld >= A + 1 (the value pre-activation is column A)");
     DeviceGuard guard(e->cfg.device);
     const int A = e->board.A;
     const int grid = blocks_for(n * 32, 256);

@@ -293,7 +293,7 @@ int dbaz_nn_stem(dbaz_engine *e, const dbaz_state *leaf_states, const float *w01
 int dbaz_nn_stem_mma_pack(dbaz_engine *e, const void *w48, void *packed, int32_t cout, uint64_t stream);
 int dbaz_nn_stem_mma(dbaz_engine *e, const dbaz_state *leaf_states, const void *packed, void *out, int32_t cout, int32_t dtype,
                      int64_t n, uint64_t stream);
-/* logits [n][ld]: columns 0..A-1 policy logits, column A value pre-activation ->
+/* logits [n][ld], ld >= A + 1: columns 0..A-1 policy logits, column A value pre-activation ->
  * priors float32[n][A] = softmax (exp(log_softmax)), values float32[n] = tanh. */
 int dbaz_nn_heads(dbaz_engine *e, const void *logits, int32_t ld, int32_t dtype, float *priors, float *values, int64_t n,
                   uint64_t stream);
