@@ -50,7 +50,6 @@ SYMBOLS = {
     "dbaz_search_reset_roots": (C.c_int, [_P, _P, _U64]),
     "dbaz_search_begin": (C.c_int, [_P, _P, _I32, _P, _D, _U64]),
     "dbaz_search_step": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _P, _P, _U64]),
-    "dbaz_search_step2": (C.c_int, [_P, _I32, _I32, _I32, _P, _P, _P, _I32, _I32, _P, _U64]),
     "dbaz_search_loop_build": (C.c_int, [_P, _P, _P, _P, _I32, _I32, C.c_float, C.c_float, C.c_float, C.c_float, _P]),
     "dbaz_search_loop_pick": (C.c_int, [_P, _P, _I32, C.c_float, C.c_float, C.c_float, _I32]),
     "dbaz_search_loop_launch": (C.c_int, [_P, _U64, _U64]),
@@ -73,7 +72,6 @@ SYMBOLS = {
     "dbaz_search_set_batch_rows": (C.c_int, [_P, _I32]),
     "dbaz_cache_configure": (C.c_int, [_P, _I32]),
     "dbaz_cache_clear": (C.c_int, [_P, _U64]),
-    "dbaz_nn_epilogue": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _I32, _I32, _I32, _U64]),
     "dbaz_nn_stem": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I32, _I32, _I32, _I64, _U64]),
     "dbaz_nn_stem_mma_pack": (C.c_int, [_P, _P, _P, _I32, _U64]),
     "dbaz_nn_stem_mma": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I64, _U64]),

@@ -2,7 +2,6 @@
 // Plain pointers and sizes only; no torch types.  Built in-tree for sm_100a:
 //   nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -shared -Xcompiler -fPIC ...
 #include <algorithm>
-#include <numeric>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -241,7 +240,6 @@ int dbaz_engine_create(const dbaz_config* cfg, dbaz_engine** out) {
     cudaMemset(ta.ctr, 0, 16 * sizeof(int));
     cudaMemset(ta.path_wn, 0, (size_t)ta.n_trees * PATH_CAP * sizeof(uint2));
     ta.batch_rows = 0x7fffffff;
-    ta.phase = 0; ta.buf = 0;
     ta.cache_vcell = C;  // action C = horizontal edge (row 0, column C): always a padding cell
     cudaMemset(ta.path, 0, (size_t)max_pending * ta.n_trees * PATH_CAP * sizeof(uint32_t));
     // an all-empty-board root set so that the engine is usable right after create
@@ -355,45 +353,6 @@ int dbaz_fake_nn(dbaz_engine* e, const dbaz_state* leaf_states, float* priors, f
 }
 
 /* ------------------------------------------------- leaf-eval fused stages */
-
-int dbaz_nn_epilogue(dbaz_engine* e, void* x, const void* res, const float* bias, const float* scale, const float* shift,
-                     int64_t rows, int32_t channels, int32_t dtype, int32_t mode, uint64_t stream) {
-    if (!e || !x || !scale || !shift) return 1;
-    if (mode < 0 || mode > 2) return fail(e, "bad epilogue mode");
-    if (rows <= 0) return 0;
-    DeviceGuard guard(e->cfg.device);
-    const int per = dtype == DBAZ_F32 ? 4 : 8;
-    if (dtype != DBAZ_F32 && dtype != DBAZ_BF16 && dtype != DBAZ_F16) return fail(e, "bad dtype");
-    if (channels % per) return fail(e, "channels must be a multiple of the vector width");
-    const int cv = channels / per;
-    const int64_t n_vec64 = rows * cv;
-    if (n_vec64 >= (int64_t)1 << 31) return fail(e, "epilogue tensor too large");
-    const uint32_t n_vec = (uint32_t)n_vec64;
-    // total threads must be a multiple of cv so that each thread owns a fixed channel group
-    int block = 256;
-    while (block % cv && block > 32) block >>= 1;
-    int64_t want = std::min<int64_t>((n_vec + (int64_t)block * 4 - 1) / ((int64_t)block * 4), (int64_t)e->n_sms * 8);
-    int grid = (int)std::max<int64_t>(want, 1);
-    if ((int64_t)block % cv) {  // cv does not divide the block: make the grid supply the multiple
-        int g = cv / std::__gcd(cv, block);
-        grid = (grid + g - 1) / g * g;
-    }
-#define DBAZ_EPI(KERNEL, TYPE)                                                                                     \
-    do {                                                                                                           \
-        if (mode == 0) KERNEL<TYPE, 0><<<grid, block, 0, S(stream)>>>((TYPE*)x, (const TYPE*)res, bias, scale, shift, n_vec, channels); \
-        else if (mode == 1) KERNEL<TYPE, 1><<<grid, block, 0, S(stream)>>>((TYPE*)x, (const TYPE*)res, bias, scale, shift, n_vec, channels); \
-        else KERNEL<TYPE, 2><<<grid, block, 0, S(stream)>>>((TYPE*)x, (const TYPE*)res, bias, scale, shift, n_vec, channels); \
-    } while (0)
-    if (dtype == DBAZ_BF16) DBAZ_EPI(k_nn_epilogue16, __nv_bfloat16);
-    else if (dtype == DBAZ_F16) DBAZ_EPI(k_nn_epilogue16, __half);
-    else {
-        if (mode == 0) k_nn_epilogue32<0><<<grid, block, 0, S(stream)>>>((float*)x, (const float*)res, bias, scale, shift, n_vec, channels);
-        else if (mode == 1) k_nn_epilogue32<1><<<grid, block, 0, S(stream)>>>((float*)x, (const float*)res, bias, scale, shift, n_vec, channels);
-        else k_nn_epilogue32<2><<<grid, block, 0, S(stream)>>>((float*)x, (const float*)res, bias, scale, shift, n_vec, channels);
-    }
-#undef DBAZ_EPI
-    return launch_ok(e, "k_nn_epilogue");
-}
 
 int dbaz_nn_stem(dbaz_engine* e, const dbaz_state* leaf_states, const float* w01, const float* bias_pos, const float* k2_pos,
                  const float* scale, const float* shift, void* out, int32_t cout, int32_t dtype, int32_t mode, int64_t n,
@@ -546,23 +505,6 @@ int dbaz_search_step(dbaz_engine* e, const float* priors, const float* values, v
         DBAZ_DISPATCH(e, (k_search_step<APL, NW, false><<<grid, TREE_WARPS * 32, 0, S(stream)>>>(
                              e->board, e->ta, e->pending, priors, values, e->noise, e->coeff, planes, dtype, layout, leaf_states, leaf_kind)));
     return launch_ok(e, "k_search_step");
-}
-
-int dbaz_search_step2(dbaz_engine* e, int32_t phase, int32_t buf, int32_t max_inline, const float* priors, const float* values, void* planes,
-                      int32_t dtype, int32_t layout, dbaz_state* leaf_states, uint64_t stream) {
-    if (!e || !planes || !leaf_states) return 1;
-    if (phase != 1 && phase != 2) return fail(e, "dbaz_search_step2: phase must be 1 (absorb) or 2 (chain)");
-    if (phase == 1 && (!priors || !values)) return 1;
-    if (buf < 0 || buf > 1 || max_inline < 0) return fail(e, "dbaz_search_step2: bad batch index / max_inline");
-    if (e->pending != 1 || !e->ta.compact) return fail(e, "dbaz_search_step2 needs max_pending_evals == 1 and compact rows (dbaz_search_set_mode)");
-    if (dtype < DBAZ_F32 || dtype > DBAZ_I16 || layout < 0 || layout > 1) return fail(e, "bad dtype/layout");
-    DeviceGuard guard(e->cfg.device);
-    TreeArgs ta = e->ta;
-    ta.phase = phase; ta.buf = buf; ta.max_inline = max_inline;
-    const int grid = blocks_for(ta.n_trees, TREE_WARPS);
-    DBAZ_DISPATCH(e, (k_search_step<APL, NW, true><<<grid, TREE_WARPS * 32, 0, S(stream)>>>(
-                         e->board, ta, 1, priors, values, e->noise, e->coeff, planes, dtype, layout, leaf_states, nullptr)));
-    return launch_ok(e, "k_search_step (phase)");
 }
 
 /* ---------------------------------------------------------- one graph per search */

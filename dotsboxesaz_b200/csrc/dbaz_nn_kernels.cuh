@@ -1,7 +1,6 @@
-// dbaz_nn_kernels.cuh -- fused elementwise stages of the leaf-evaluation pipeline.  The dense
-// contractions (conv / linear) stay in cuDNN / cuBLAS; everything between them that PyTorch
-// eager would run as 3-4 separate passes (bias add, ReLU, eval-mode BatchNorm, dtype casts,
-// log-softmax + exp, tanh) is one HBM pass here.
+// dbaz_nn_kernels.cuh -- fused stages of the leaf-evaluation pipeline.  The heads (log-softmax +
+// exp, tanh) are one HBM pass here instead of PyTorch eager's several; the stem gathers the leaves
+// and runs the first convolution with its bias / ReLU / eval-mode BatchNorm in one kernel.
 //
 // Reference semantics: dots_boxes/dots_boxes_nn.py:85-98 (x = bn(relu(conv(x)))), nn.py:49-58,
 // nn.py:155-160 (p = exp(log_softmax), v = tanh).
@@ -39,95 +38,6 @@ template <> struct Vec8<__half> {
         for (int i = 0; i < 4; ++i) h[i] = __floats2half2_rn(f[2 * i], f[2 * i + 1]);
     }
 };
-
-// mode 0:  y = scale[c] * relu(x + bias[c]) + shift[c]            (SimpleNN: conv -> ReLU -> BN)
-// mode 1:  y = relu(scale[c] * (x + bias[c]) + shift[c] + res)    (ResNetZero: conv -> BN -> (+res) -> ReLU), res may be null
-// mode 2:  y = scale[c] * (x + bias[c]) + shift[c]                (affine only)
-// x is [rows, C] with the channel innermost (NHWC conv output / linear output), in place.
-//
-// HBM-bound: one 16-byte vector (VW channels) per thread per iteration.  The host sizes the grid so
-// that the total thread count is a multiple of C/VW: a thread then always sees the same VW channels and
-// keeps their bias/scale/shift in registers for the whole grid-stride loop (the per-element parameter
-// loads and the 64-bit modulo of a naive version made it LSU-bound at 1.5 TB/s).  UNROLL independent
-// vectors are in flight per thread.
-template <int MODE>
-__device__ __forceinline__ float epi_apply(float x, float b, float s, float t, float r, bool has_res) {
-    float y = x + b;
-    if (MODE == 0) return fmaf(s, fmaxf(y, 0.0f), t);
-    if (MODE == 1) { y = fmaf(s, y, t); if (has_res) y += r; return fmaxf(y, 0.0f); }
-    return fmaf(s, y, t);
-}
-
-template <typename T, int MODE>
-__global__ void __launch_bounds__(256)
-k_nn_epilogue16(T* __restrict__ x, const T* __restrict__ res, const float* __restrict__ bias,
-                const float* __restrict__ scale, const float* __restrict__ shift, uint32_t n_vec, int C) {
-    constexpr int UNROLL = 4;
-    const uint32_t nthreads = gridDim.x * blockDim.x, tid = blockIdx.x * blockDim.x + threadIdx.x;
-    const int c0 = (int)(tid % (uint32_t)(C >> 3)) << 3;
-    float b[8], s[8], t[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { b[j] = bias ? bias[c0 + j] : 0.0f; s[j] = scale[c0 + j]; t[j] = shift[c0 + j]; }
-    uint4* xv = reinterpret_cast<uint4*>(x);
-    const uint4* rv = reinterpret_cast<const uint4*>(res);
-    for (uint32_t base = tid; base < n_vec; base += nthreads * UNROLL) {
-        Vec8<T> v[UNROLL], r[UNROLL];
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            uint32_t i = base + u * nthreads;
-            if (i < n_vec) { v[u].raw = xv[i]; if (res) r[u].raw = rv[i]; }
-        }
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            uint32_t i = base + u * nthreads;
-            if (i < n_vec) {
-                float f[8], g[8];
-                v[u].unpack(f);
-                if (res) r[u].unpack(g);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) f[j] = epi_apply<MODE>(f[j], b[j], s[j], t[j], res ? g[j] : 0.0f, res != nullptr);
-                v[u].pack(f);
-                xv[i] = v[u].raw;
-            }
-        }
-    }
-}
-
-// fp32 variant (4 channels per 16-byte vector)
-template <int MODE>
-__global__ void __launch_bounds__(256)
-k_nn_epilogue32(float* __restrict__ x, const float* __restrict__ res, const float* __restrict__ bias,
-                const float* __restrict__ scale, const float* __restrict__ shift, uint32_t n_vec, int C) {
-    constexpr int UNROLL = 4;
-    const uint32_t nthreads = gridDim.x * blockDim.x, tid = blockIdx.x * blockDim.x + threadIdx.x;
-    const int c0 = (int)(tid % (uint32_t)(C >> 2)) << 2;
-    float b[4], s[4], t[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { b[j] = bias ? bias[c0 + j] : 0.0f; s[j] = scale[c0 + j]; t[j] = shift[c0 + j]; }
-    float4* xv = reinterpret_cast<float4*>(x);
-    const float4* rv = reinterpret_cast<const float4*>(res);
-    for (uint32_t base = tid; base < n_vec; base += nthreads * UNROLL) {
-        float4 v[UNROLL], r[UNROLL];
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            uint32_t i = base + u * nthreads;
-            r[u] = make_float4(0, 0, 0, 0);
-            if (i < n_vec) { v[u] = xv[i]; if (res) r[u] = rv[i]; }
-        }
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            uint32_t i = base + u * nthreads;
-            if (i < n_vec) {
-                float4 o;
-                o.x = epi_apply<MODE>(v[u].x, b[0], s[0], t[0], r[u].x, res != nullptr);
-                o.y = epi_apply<MODE>(v[u].y, b[1], s[1], t[1], r[u].y, res != nullptr);
-                o.z = epi_apply<MODE>(v[u].z, b[2], s[2], t[2], r[u].z, res != nullptr);
-                o.w = epi_apply<MODE>(v[u].w, b[3], s[3], t[3], r[u].w, res != nullptr);
-                xv[i] = o;
-            }
-        }
-    }
-}
 
 // Heads: logits [n, ld] (policy logits in columns 0..A-1, value pre-activation in column A) ->
 // priors float32 [n, A] = softmax (== exp(log_softmax), nn.py:159), values float32 [n] = tanh.
@@ -210,8 +120,9 @@ namespace dbaz {
 //     y[p][co] = B[p][co] + k * K2[p][co] + sum over (plane c in {0,1}, tap inside the board, edge bit set) W01[c][tap][co]
 // where the host has folded into B / K2 / W01 (all float32, exact algebra): the conv bias, the optional
 // input BatchNorm of ResNetZero (nn.py:118; its shift only contributes through in-board taps, hence the
-// position dependence) and the third plane's weights summed over in-board taps.  The epilogue is the
-// same as k_nn_epilogue (mode 0: scale*relu(y)+shift; mode 1: relu(scale*y+shift)).
+// position dependence) and the third plane's weights summed over in-board taps.  The epilogue per output
+// channel: mode 0 scale*relu(y)+shift (SimpleNN: conv -> ReLU -> BN), mode 1 relu(scale*y+shift) (ResNetZero:
+// conv -> BN -> ReLU).
 //
 // Thread = (leaf, group of 8 output channels); all positions of a tile are accumulated in registers
 // with the tap loop outermost, so each weight vector is read from shared memory once per leaf.  H, W

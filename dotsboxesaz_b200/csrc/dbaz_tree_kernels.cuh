@@ -116,18 +116,7 @@ struct TreeArgs {
     int max_inline;       // > 0: at most this many simulations per tree and launch may finish without the net
     int chain_clk;        // > 0: ... and none is started once the tree has spent this many SM clocks in the launch
     int batch_rows;       // compact mode: rows the evaluator of this launch will run; a leaf beyond them waits a wave
-    // Overlapped chains (compact mode, dbaz_search_step2): a wave is two launches over two leaf batches 0 / 1.
-    //   phase 1 "absorb": trees whose pending leaf sits in batch buf ^ 1 (just evaluated) are backed up and run on; trees in
-    //     the middle of a chain run on too; leaves go to batch `buf` behind the ctr[8 + buf] rows phase 2 of the previous wave
-    //     put there; a tree whose leaf waits in batch `buf` (not evaluated yet) is left alone.  Publishes the wave counters.
-    //   phase 2 "chain": only trees without a pending leaf run on -- concurrently with the evaluator of batch `buf` -- and
-    //     their leaves go to batch buf ^ 1 from row 0 (row counter ctr[8 + (buf ^ 1)]).
-    //   phase 0: the single-launch wave of dbaz_search_step (batch 0 only).
-    // TreeRec.row carries the batch in bit 30.
-    int phase, buf;
 };
-constexpr int ROW_BUF_SHIFT = 30;
-constexpr int ROW_MASK = (1 << ROW_BUF_SHIFT) - 1;
 
 __device__ __forceinline__ char* node_ptr(const TreeArgs& ta, int t, int i) {
     return ta.arena + ((int64_t)t * ta.max_nodes + i) * (int64_t)ta.stride;
@@ -868,20 +857,16 @@ __device__ __forceinline__ bool search_step_seq(const Board& b, const TreeArgs& 
     // ---- one round trip: everything whose address depends only on t
     TreeHot T = load_hot(ta.trees + t);
     const bool compact = ta.compact;
-    const int phase = ta.phase;
     LaneActions<APL, NW> la;
     la.load(b, ta.act_tab, lane);
     StepInputs<APL> in;
     if (!compact) load_pending<APL, true>(b, ta, t, 0, -1, priors, values, in, lane);
-    const int row_base = (phase == 1) ? ta.ctr[8 + ta.buf] : 0;  // rows the chain launch of the previous wave already took
 
     if (T.n_pending <= 0 && T.sims_left <= 0) {  // idle tree
         if (leaf_kind && !compact && lane == 0) leaf_kind[t] = 0;
         return false;
     }
-    if (phase == 2 && T.n_pending > 0) return true;  // its leaf is with the evaluator right now
-    if (phase == 1 && T.n_pending > 0 && ((T.row >> ROW_BUF_SHIFT) & 1) == ta.buf) return true;  // ... or waits for the next evaluator call
-    if (compact) load_pending<APL, true>(b, ta, t, 0, T.n_pending > 0 ? (T.row & ROW_MASK) : 0, priors, values, in, lane);
+    if (compact) load_pending<APL, true>(b, ta, t, 0, T.n_pending > 0 ? T.row : 0, priors, values, in, lane);
     WaveStats ws = {0, 0, 0, 0, 0};
     if (T.n_pending > 0) {
         tree_expand_backup<APL, NW, true>(b, ta, t, T, in, sh, lane, EV_NET, ws);
@@ -912,10 +897,7 @@ __device__ __forceinline__ bool search_step_seq(const Board& b, const TreeArgs& 
                 int64_t row = t;
                 if (compact) {
                     int r = 0;
-                    if (lane == 0) {
-                        if (phase == 2) r = atomicAdd(&ta.ctr[8 + (ta.buf ^ 1)], 1);
-                        else r = row_base + (int)(atomicAdd(reinterpret_cast<unsigned long long*>(ta.ctr), 1ull << 40) >> 40);
-                    }
+                    if (lane == 0) r = (int)(atomicAdd(reinterpret_cast<unsigned long long*>(ta.ctr), 1ull << 40) >> 40);
                     r = __shfl_sync(0xffffffffu, r, 0);
                     if (r >= ta.batch_rows) {
                         // the evaluator's batch is full: this selection is dropped and repeated in the next wave.
@@ -924,7 +906,7 @@ __device__ __forceinline__ bool search_step_seq(const Board& b, const TreeArgs& 
                         T.sims_left += 1;
                         break;
                     }
-                    T.row = r | ((phase == 2 ? (ta.buf ^ 1) : (phase == 1 ? ta.buf : 0)) << ROW_BUF_SHIFT);
+                    T.row = r;
                     row = r;
                 }
                 emit_leaf<APL, NW, true>(b, ta, in, t, row, planes, dtype, layout, leaf_states, lane);
@@ -1031,7 +1013,7 @@ __device__ __forceinline__ bool search_step_waves(const Board& b, const TreeArgs
 // own register allocation and half the code.
 template <int APL, int NW, bool SEQ>
 // Resident trees per SM (= register cap): 28 -> 72 registers for one action per lane (3x3), 20 -> 102 for two; for three and
-// more (5x5: 168 registers uncapped, 12 trees per SM, 13 % of the warp slots) 16 -> 128 registers with 36 bytes of spills:
+// more (5x5: 168 registers uncapped, 12 trees per SM, 13 % of the warp slots) 16 -> 128 registers, even where that spills:
 // the kernel is latency-bound with nine waves of CTAs, so residency wins -- 139 -> 114 us per launch on configs[3] (20 -> 96
 // registers: 111 us, 156 bytes of spills).
 __global__ void __launch_bounds__(TREE_WARPS * 32, (APL == 1 ? 28 : (APL == 2 ? 20 : 16)) / TREE_WARPS)
@@ -1054,17 +1036,16 @@ k_search_step(Board b, TreeArgs ta, int pending /* max_pending_evals of this sea
     // ---- wave bookkeeping, per warp (no CTA barrier: a warp leaves as soon as its tree is done, so a long chain keeps
     // one warp slot busy, not four).  Rows asked for, busy trees and finished warps share ONE 64-bit word, so a single
     // atomic per warp keeps them consistent without a fence; the warp that completes the count publishes and re-arms.
-    if (lane == 0 && ta.phase != 2) {  // the chain launch (phase 2) publishes nothing: the next absorb launch counts its rows
+    if (lane == 0) {
         unsigned long long* word = reinterpret_cast<unsigned long long*>(ta.ctr);
         const unsigned long long inc = 1ull | (busy ? (1ull << 20) : 0ull);
         const unsigned long long now = atomicAdd(word, inc) + inc;
         if ((now & 0xfffffull) == (unsigned long long)(gridDim.x * TREE_WARPS)) {
-            const int rows = (int)(now >> 40) + (ta.phase == 1 ? ta.ctr[8 + ta.buf] : 0);
+            const int rows = (int)(now >> 40);
             ta.ctr[4] = rows;
             ta.ctr[5] = (int)((now >> 20) & 0xfffffull);
             if (rows > ta.ctr[6]) ta.ctr[6] = rows;
             *word = 0ull;  // nobody else touches it before the next launch
-            if (ta.phase == 1) ta.ctr[8 + (ta.buf ^ 1)] = 0;  // the batch just absorbed: the chain launch fills it from row 0
         }
     }
 }

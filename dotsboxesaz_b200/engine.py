@@ -55,25 +55,15 @@ class Engine:
         # search I/O buffers (fixed addresses, so the wave loop can be captured in a CUDA graph).  One row per
         # in-flight simulation: row of slot k of tree t = k * n_games + t; a search with max_pending_evals = K uses
         # the first K * n_games rows (`self.n_rows`), evaluators work on the `[:n_rows]` views below.
-        # Two leaf batches: the overlapped wave loop (step2) alternates between them -- the evaluator works on one while
-        # the chain launch already fills the other; everything else uses batch 0 (`self._buf`).
         cap = n_games * self.max_pending
-        self._priors2 = torch.zeros((2, cap, self.A), dtype=torch.float32, device=self.device)
-        self._values2 = torch.zeros((2, cap), dtype=torch.float32, device=self.device)
-        self._leaf_states2 = torch.zeros((2, cap, 4), dtype=torch.int64, device=self.device)
+        self._priors = torch.zeros((cap, self.A), dtype=torch.float32, device=self.device)
+        self._values = torch.zeros((cap,), dtype=torch.float32, device=self.device)
+        self._leaf_states = torch.zeros((cap, 4), dtype=torch.int64, device=self.device)
         self._leaf_kind = torch.zeros((cap,), dtype=torch.int8, device=self.device)
-        self._buf = 0
-        # Optional: the adaptive wave loop as two launches per wave (step2), chains of evaluator-free simulations continuing
-        # on a second stream under the evaluator.  Bit-identical results (tests/test_gpu_cache.py), but measured SLOWER on
-        # B200 (configs[1]: 25.2 vs 27.9 M sims/s -- the chain launch takes SM slots from the evaluator and the fork/join costs
-        # more per wave than the hidden part of the step kernel saves; DESIGN.md section 3), hence off by default.
-        self.overlap = os.environ.get("DBAZ_OVERLAP", "0") == "1"
-        self.chain_inline = 16       # ... and may be this long per wave (they cost nothing on the critical path)
-        self._side = None            # the second stream of the overlapped loop
         self.pending = 1
         self._batch_rows = None      # evaluator batch of the adaptive wave loop (None: pending * n_games)
-        self._planes2 = None
-        self._planes_base2 = None
+        self._planes = None
+        self._planes_base = None
         self._plane_cfg = None
         self._noise = None  # keeps the caller's noise buffer alive while the engine may read it
         self._num_reads = torch.zeros((n_games,), dtype=torch.int32, device=self.device)
@@ -221,18 +211,6 @@ class Engine:
         return int(buf[0]), int(buf[1])
 
     @property
-    def _priors(self):
-        return self._priors2[self._buf]
-
-    @property
-    def _values(self):
-        return self._values2[self._buf]
-
-    @property
-    def _leaf_states(self):
-        return self._leaf_states2[self._buf]
-
-    @property
     def priors(self):
         return self._priors[:self.n_rows]
 
@@ -249,14 +227,6 @@ class Engine:
         return self._leaf_kind[:self.n_rows]
 
     @property
-    def _planes(self):
-        return self._planes2[self._buf]
-
-    @property
-    def _planes_base(self):
-        return self._planes_base2[self._buf]
-
-    @property
     def planes(self):
         return self._planes[:self.n_rows]
 
@@ -266,12 +236,12 @@ class Engine:
         if cfg != self._plane_cfg:
             cap = self.n_games * self.max_pending
             if channels_last:
-                base = torch.zeros((2, cap, self.rows, self.cols, 3), dtype=dtype, device=self.device)
-                self._planes2 = base.permute(0, 1, 4, 2, 3)  # logical NCHW view over NHWC memory
-                self._planes_base2 = base
+                base = torch.zeros((cap, self.rows, self.cols, 3), dtype=dtype, device=self.device)
+                self._planes = base.permute(0, 3, 1, 2)  # logical NCHW view over NHWC memory
+                self._planes_base = base
             else:
-                self._planes2 = torch.zeros((2, cap, 3, self.rows, self.cols), dtype=dtype, device=self.device)
-                self._planes_base2 = self._planes2
+                self._planes = torch.zeros((cap, 3, self.rows, self.cols), dtype=dtype, device=self.device)
+                self._planes_base = self._planes
             self._plane_cfg = cfg
         return self.planes
 
@@ -354,15 +324,6 @@ class Engine:
         return priors, values
 
     # ------------------------------------------------- leaf-eval fused stages
-    def nn_epilogue(self, x, bias, scale, shift, mode=0, res=None):
-        """In place on x ([..., channels] contiguous, channel innermost): mode 0 scale*relu(x+bias)+shift,
-        mode 1 relu(scale*(x+bias)+shift(+res)), mode 2 scale*(x+bias)+shift (include/dbaz_b200.h)."""
-        ch = x.shape[-1]
-        rows = x.numel() // ch
-        self._ck(self.lib.dbaz_nn_epilogue(self._h, _ptr(x), _ptr(res), _ptr(bias), _ptr(scale), _ptr(shift), rows, ch,
-                                           _DTYPE_CODE[x.dtype], int(mode), self._stream()))
-        return x
-
     def nn_stem(self, leaf_states, w01, bias_pos, k2_pos, scale, shift, out, mode=0):
         """Leaf gather + first 3x3 conv + epilogue in one kernel, from packed states (include/dbaz_b200.h).
         out: [n, L+1, C+1, cout] contiguous (NHWC), bf16/fp16."""
@@ -478,17 +439,6 @@ class Engine:
                                            _DTYPE_CODE[dtype], _capi.NHWC if cl else _capi.NCHW, _ptr(self._leaf_states),
                                            _ptr(self._leaf_kind), self._stream()))
         self._nw += 1
-
-    def step2(self, phase, buf, max_inline):
-        """One launch of the two-launch wave (include/dbaz_b200.h: dbaz_search_step2).  phase 1 absorbs batch buf ^ 1 and
-        fills batch `buf`; phase 2 continues evaluator-free chains and fills batch buf ^ 1."""
-        dtype, cl = self._plane_cfg
-        src, dst = (buf ^ 1, buf) if phase == 1 else (buf, buf ^ 1)
-        self._ck(self.lib.dbaz_search_step2(self._h, int(phase), int(buf), int(max_inline), _ptr(self._priors2[src]), _ptr(self._values2[src]),
-                                            _ptr(self._planes_base2[dst]), _DTYPE_CODE[dtype], _capi.NHWC if cl else _capi.NCHW,
-                                            _ptr(self._leaf_states2[dst]), self._stream()))
-        if phase == 1:
-            self._nw += 1
 
     def step_flush(self):
         """Stop launching simulations (UCT_search's time limit) and back up the pending leaves."""
@@ -662,7 +612,7 @@ class Engine:
         """{batch rows: CUDA graph of `graph_waves` [step -> evaluator] waves} for every rung of the ladder (compact mode).
         Every batch size is captured up front: capturing re-binds the search head and idles all trees."""
         key = (id(evaluator), graph_waves, noise is not None, float(coeff), self._plane_cfg, 1, self._mode_key(), "ladder", self.LADDER_STEPS,
-               short_tail, tuple(self._ladder(evaluator)), bool(self.overlap), int(self.chain_inline))
+               short_tail, tuple(self._ladder(evaluator)))
         if key not in self._graphs:
             graphs = {}
             for rows in self._ladder(evaluator):
@@ -678,10 +628,7 @@ class Engine:
     def _rung_waves(self, rows, graph_waves):
         """Waves per graph replay of a rung: the small rungs run at the end of a search, where the host's decision lag
         (two replays) is pure overhead once the last tree has finished, so their graphs are shorter."""
-        w = max(1, graph_waves // 4) if rows * 8 <= self.n_games else graph_waves
-        if self.overlap and graph_waves >= 2:
-            w = max(2, w - (w & 1))  # the overlapped loop alternates two leaf batches and every graph starts on batch 0
-        return w
+        return max(1, graph_waves // 4) if rows * 8 <= self.n_games else graph_waves
 
     def _pick_rows(self, ladder, want, ev_id):
         """The batch size for waves that are expected to ask for `want` rows: the rung that holds them and serves the most
@@ -772,34 +719,10 @@ class Engine:
         self.lib.dbaz_search_begin(self._h, _ptr(self._idle_reads), int(pending), _ptr(noise), float(coeff), self._stream())
         g = torch.cuda.CUDAGraph(keep_graph=True) if self._batch_rows is not None else torch.cuda.CUDAGraph()
         n0, w0 = self._nl, self._nw
-        overlapped = bool(self.overlap and self.compact and int(pending) == 1 and graph_waves >= 2 and graph_waves % 2 == 0)
-        if overlapped and self._side is None:
-            self._side = torch.cuda.Stream(device=self.device)
         with torch.cuda.graph(g, pool=self._graph_pool):
-            if not overlapped:
-                for _ in range(graph_waves):
-                    self.step()
-                    evaluator(self)
-            else:
-                # wave w works on leaf batch w & 1: [absorb batch b ^ 1, fill batch b] -> evaluator(batch b) on this stream,
-                # the chains of evaluator-free simulations (filling batch b ^ 1) on the side stream at the same time.
-                # Nothing is carried across graphs: the last wave has no chain launch, every graph starts on batch 0.
-                main = torch.cuda.current_stream(self.device)
-                chain_inline = int(self.chain_inline)  # extra evaluator-free simulations per wave, off the critical path
-                for w in range(graph_waves):
-                    b = w & 1
-                    self._buf = b
-                    self.step2(1, b, int(inline))  # the usual budget: a chain that ends inside it still makes THIS wave's batch
-                    chain = w + 1 < graph_waves
-                    if chain:
-                        self._side.wait_stream(main)
-                        with torch.cuda.stream(self._side):
-                            self.step2(2, b, chain_inline)
-                    evaluator(self)
-                    if chain:
-                        main.wait_stream(self._side)
-                self._buf = 0
-        self._buf = 0
+            for _ in range(graph_waves):
+                self.step()
+                evaluator(self)
         self._graph_cost[id(g)] = (self._nl - n0, self._nw - w0)  # engine kernels / waves one replay stands for
         self._nl, self._nw = n0, w0  # capture enqueues nothing
         self.lib.dbaz_search_set_batch_rows(self._h, 0)

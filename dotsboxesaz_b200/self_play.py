@@ -368,16 +368,15 @@ class BatchedSelfPlay:
         fgraph = torch.cuda.CUDAGraph()
         l0 = eng.n_launches
         main = torch.cuda.current_stream(dev)
-        if eng._side is None:
-            eng._side = torch.cuda.Stream(device=dev)
-        eng._side.wait_stream(main)
-        with torch.cuda.stream(eng._side):
+        side = torch.cuda.Stream(device=dev)
+        side.wait_stream(main)
+        with torch.cuda.stream(side):
             fgraph.capture_begin()
             try:
                 finish()
             finally:
                 fgraph.capture_end()
-        main.wait_stream(eng._side)
+        main.wait_stream(side)
         finish_launches = eng.n_launches - l0  # engine kernels inside the finish graph
         eng.n_launches = l0
         stream = torch.cuda.current_stream(dev)

@@ -129,22 +129,6 @@ int dbaz_search_begin(dbaz_engine *e, const int32_t *num_reads, int32_t pending,
  *   never appear: their simulation is completed inside the step, as in the reference where it never awaits. */
 int dbaz_search_step(dbaz_engine *e, const float *priors, const float *values, void *planes, int32_t dtype,
                      int32_t layout, dbaz_state *leaf_states, int8_t *leaf_kind, uint64_t stream);
-/* The same wave as TWO launches, so that the part of it that needs no evaluator runs UNDER the evaluator
- * (max_pending_evals == 1, compact rows; two leaf batches 0 / 1 that alternate from wave to wave):
- *   phase 1 "absorb" (before the evaluator of batch `buf`): trees whose pending leaf sits in batch buf ^ 1 -- evaluated by the
- *     previous wave, priors / values point at THAT batch -- are backed up and run on as in dbaz_search_step; trees in the
- *     middle of a chain of evaluator-free simulations (terminal leaves, eval-cache hits) run on too; at most `max_inline`
- *     such simulations complete per tree; leaves go to batch `buf` (planes / leaf_states point at it) behind the rows
- *     phase 2 of the previous wave put there; a tree whose leaf already waits in batch `buf` is left alone.  Publishes the
- *     wave counters (dbaz_search_wave_counts).
- *   phase 2 "chain" (a second stream, concurrently with the evaluator of batch `buf`): only trees WITHOUT a pending leaf run
- *     on, up to `max_inline` completions, and their leaves go to batch buf ^ 1 from row 0 (planes / leaf_states point at
- *     batch buf ^ 1; priors / values are not read).
- * The order of a tree's simulations is untouched, so every result equals dbaz_search_step's.  A sequence of waves must
- * start with buf = 0, alternate, and end with a phase 1 that no phase 2 follows (nothing is carried across sequences). */
-int dbaz_search_step2(dbaz_engine *e, int32_t phase, int32_t buf, int32_t max_inline, const float *priors,
-                      const float *values, void *planes, int32_t dtype, int32_t layout, dbaz_state *leaf_states,
-                      uint64_t stream);
 /* UCT_search's wall-clock limit (mcts.py:201-203,232-233): no tree starts another simulation; the
  * next dbaz_search_step() only backs up the leaves already pending. */
 int dbaz_search_stop(dbaz_engine *e, uint64_t stream);
@@ -266,15 +250,10 @@ int dbaz_cache_configure(dbaz_engine *e, int32_t log2_entries);
 /* Forget every entry (call after the net's weights change).  O(1): the keys carry a table epoch, which this call bumps. */
 int dbaz_cache_clear(dbaz_engine *e, uint64_t stream);
 
-/* ---- leaf-evaluation pipeline: fused elementwise stages between the library GEMMs/convs ----
- * (replaces the separate bias / ReLU / eval-BatchNorm / softmax passes of NeuralNetWrapper.predict_sync,
- * nn.py:155-160, around dots_boxes_nn.py:85-98 and nn.py:49-58).  x: [rows, channels], channel innermost
- * (NHWC conv output or linear output), updated in place; bias may be NULL; scale/shift are the folded
- * eval-mode BatchNorm (gamma/sqrt(var+eps), beta - mean*scale), float32[channels].
- *   mode 0: y = scale*relu(x+bias)+shift      mode 1: y = relu(scale*(x+bias)+shift (+res))
- *   mode 2: y = scale*(x+bias)+shift */
-int dbaz_nn_epilogue(dbaz_engine *e, void *x, const void *res, const float *bias, const float *scale, const float *shift,
-                     int64_t rows, int32_t channels, int32_t dtype, int32_t mode, uint64_t stream);
+/* ---- leaf-evaluation pipeline: fused stages around the library GEMMs/convs ----
+ * (replace the separate gather / bias / ReLU / eval-BatchNorm / softmax passes of NeuralNetWrapper.predict_sync,
+ * nn.py:155-160, around dots_boxes_nn.py:85-98 and nn.py:49-58).  scale/shift are the folded eval-mode BatchNorm
+ * (gamma/sqrt(var+eps), beta - mean*scale), float32[channels]. */
 /* Leaf gather + first 3x3 conv (zero padding 1, 3 input planes) + epilogue in one kernel, reading the packed
  * leaf states instead of a plane tensor (dots_boxes_game.py:96-100 + dots_boxes_nn.py:85 / nn.py:118-119,27-28).
  * w01 float32[2][3][3][cout]: weights of the two edge planes; bias_pos / k2_pos float32[(L+1)*(C+1)][cout]:

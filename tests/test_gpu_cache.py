@@ -65,14 +65,14 @@ def _play(eng, ev, roots, sims, moves, noise_seed, **kw):
     return out
 
 
-@pytest.mark.parametrize("overlap", [False, True])
+@pytest.mark.parametrize("device_loop", [True, False], ids=["device_loop", "host_loop"])
 @pytest.mark.parametrize("board,n,sims,log2,max_inline,margin", [((3, 3), 192, 300, 14, 0, 1.125), ((3, 3), 192, 300, 5, 2, 1.125),
                                                                  ((5, 5), 96, 200, 12, 0, 1.125), ((2, 3), 64, 150, 10, 3, 1.125),
                                                                  ((3, 3), 512, 300, 14, 4, 0.4), ((5, 5), 256, 200, 12, 2, 0.25)])
-def test_cache_compact_adaptive_bit_exact(mods, board, n, sims, log2, max_inline, margin, overlap):
+def test_cache_compact_adaptive_bit_exact(mods, board, n, sims, log2, max_inline, margin, device_loop):
     """margin < 1 sizes the evaluator's batch BELOW what the waves ask for, so leaves overflow the batch all the time and
-    their selections are dropped and repeated (dbaz_search_set_batch_rows).  overlap: the same loop as two launches per
-    wave (dbaz_search_step2), chains of evaluator-free simulations on a second stream under the evaluator, two leaf batches."""
+    their selections are dropped and repeated (dbaz_search_set_batch_rows).  device_loop: the adaptive loop as one
+    conditional graph per search, or driven by the host (the fallback where a driver cannot build that graph)."""
     engine, oracle = mods
     ev = engine.FakeNetEvaluator(0)
     plain = engine.Engine(board, n_games=n, max_nodes=4 * sims + 64)
@@ -84,10 +84,9 @@ def test_cache_compact_adaptive_bit_exact(mods, board, n, sims, log2, max_inline
     eng = engine.Engine(board, n_games=n, max_nodes=4 * sims + 64, eval_cache=log2)
     eng.set_mode(False, max_inline)
     eng.ROW_MARGIN = margin
-    eng.overlap = overlap
-    eng.chain_inline = 3 if max_inline else 0
+    eng.device_loop = device_loop
     got = _play(eng, ev, roots.clone(), sims, 4, noise_seed=3, graph_waves=4, adaptive=True)
-    assert (eng._side is not None) == overlap
+    assert eng.device_loop == device_loop  # the conditional graph was built, not replaced by the host loop
     info = eng.status()
     for m, (a, b) in enumerate(zip(ref, got)):
         _same(a, b, (board, "move", m))

@@ -286,19 +286,16 @@ def test_batched_search_vs_oracle(mods, board, pending, kind):
         eng.close()
 
 
-@pytest.mark.parametrize("board,overlap,device_loop", [((6, 6), False, True), ((7, 7), True, True), ((7, 7), False, False),
-                                                       ((6, 6), True, False)])
-def test_production_schedule_vs_oracle(mods, board, overlap, device_loop):
+@pytest.mark.parametrize("board,device_loop", [((6, 6), True), ((7, 7), True), ((7, 7), False), ((6, 6), False)])
+def test_production_schedule_vs_oracle(mods, board, device_loop):
     """The schedule self-play runs with -- eval cache (keys split across cells past 88 actions), compact rows, in-kernel
-    chains bounded by count and time, optionally the two-launch overlapped wave (dbaz_search_step2), the adaptive batch
-    ladder and the device-driven WHILE/SWITCH loop -- checked tree by tree against the oracle itself."""
+    chains bounded by count and time, the adaptive batch ladder, driven by the device's WHILE/SWITCH loop or by the
+    host -- checked tree by tree against the oracle itself."""
     engine, oracle = mods
     n, sims = 128, 150
     eng = engine.Engine(board, n_games=n, max_nodes=4 * sims + 64, eval_cache=12)
     try:
         eng.set_mode(False, 2)
-        eng.overlap = overlap
-        eng.chain_inline = 3
         eng.device_loop = device_loop
         rng = np.random.RandomState(17 + board[0])
         st, og = _roots(eng, oracle, n, rng, max_frac=0.6)
@@ -317,17 +314,16 @@ def test_production_schedule_vs_oracle(mods, board, overlap, device_loop):
                 if term[g]:
                     continue
                 trees[g].search(int(reads[g]), noise=noise[g], coeff=0.25)
-                _check_tree(eng, snap, g, trees[g], (board, overlap, device_loop, move_i))
+                _check_tree(eng, snap, g, trees[g], (board, device_loop, move_i))
             moves = _pick_moves(trees, move_i)
             for g in range(n):
                 if moves[g] >= 0:
                     trees[g].reroot(int(moves[g]), True)
             eng.advance_roots(moves, reuse=True)
-        _check_root_states(eng, trees, (board, overlap, device_loop, "root"))
+        _check_root_states(eng, trees, (board, device_loop, "root"))
         info = eng.status()
         assert info["errors"] == 0 and info["cache_hits"] > 0
         assert eng.device_loop == device_loop       # the conditional graph was built, not replaced by the host loop
-        assert (eng._side is not None) == overlap
         assert eng.wave_counts() == (0, 0)
     finally:
         eng.close()

@@ -1,5 +1,5 @@
 """GPU numerics of the leaf-evaluation pipeline: fused inference plans (library convs/GEMMs + the
-engine's fused epilogue / heads kernels) against the plain PyTorch fp32 modules in eval mode.
+engine's stem / heads kernels) against the plain PyTorch fp32 modules in eval mode.
 Tolerances: fp32 plan 2e-5 abs on probabilities/values (north_star: Q/priors within 1e-5 relative is
 for the TREE given identical net outputs; the net itself is floating point and its plan re-associates
 sums); bf16 plans: BF16_BOUNDS below (relative error of every prior above 1e-3, per-row KL, tanh value) against the
@@ -152,36 +152,6 @@ def test_fused_plans_match_torch_modules(net, board, blocks):
             eng.planes.copy_(x32.to(dtype))
             ev(eng)
             check("module " + dn, dtype)
-    eng.close()
-
-
-@pytest.mark.parametrize("dtype", ["bf16", "fp32"])
-def test_epilogue_kernel_matches_torch(dtype):
-    """dbaz_nn_epilogue (bias + ReLU + eval-BatchNorm in one pass; the three modes of include/dbaz_b200.h) against the
-    same expression in PyTorch fp32.  Tolerance: one rounding of the storage dtype (bf16: 2^-8 relative)."""
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    from dotsboxesaz_b200 import engine
-    dt = torch.bfloat16 if dtype == "bf16" else torch.float32
-    eng = engine.Engine((3, 3), n_games=4, max_nodes=8)
-    g = torch.Generator(device="cuda").manual_seed(0)
-    rows, ch = 1000, 64
-    x = torch.randn(rows, ch, device="cuda", generator=g)
-    res = torch.randn(rows, ch, device="cuda", generator=g)
-    bias, scale, shift = (torch.randn(ch, device="cuda", generator=g) for _ in range(3))
-    for mode in (0, 1, 2):
-        for use_res in ((False, True) if mode == 1 else (False,)):
-            xr, rr = x.to(dt).float(), res.to(dt).float()
-            if mode == 0:
-                ref = scale * torch.relu(xr + bias) + shift
-            elif mode == 1:
-                ref = torch.relu(scale * (xr + bias) + shift + (rr if use_res else 0))
-            else:
-                ref = scale * (xr + bias) + shift
-            y = x.to(dt).clone()
-            eng.nn_epilogue(y, bias, scale, shift, mode=mode, res=res.to(dt) if use_res else None)
-            tol = 2 ** -7 if dtype == "bf16" else 1e-5
-            assert ((y.float() - ref).abs() <= tol * (1 + ref.abs())).all(), (dtype, mode, use_res)
     eng.close()
 
 
