@@ -83,6 +83,9 @@ SYMBOLS = {
     "dbaz_nn_tower": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _P, _I64, _U64]),
     "dbaz_nn_tower_trace": (C.c_int, [_P, _P]),
     "dbaz_fake_nn": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _U64]),
+    "dbaz_solver_solve": (C.c_int, [_P, _P, _I64, _U64]),
+    "dbaz_solver_moves": (C.c_int, [_P, _P, _P, _P, _P, _I64, _U64]),
+    "dbaz_solver_eval": (C.c_int, [_P, _P, _P, _P, _P, _I32, _I64, _U64]),
 }
 
 _lib = None

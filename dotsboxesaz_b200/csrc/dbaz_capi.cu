@@ -15,6 +15,7 @@
 #include "dbaz_selfplay.cuh"
 #include "dbaz_tower.cuh"
 #include "dbaz_loop.cuh"
+#include "dbaz_solver.cuh"
 
 using namespace dbaz;
 
@@ -35,6 +36,8 @@ struct dbaz_engine {
     unsigned long long* d_status;
     int* d_tower_err;     // set by k_resnet_tower when a barrier wait times out
     long long* tower_dbg; // caller-owned timeline buffer (dbaz_nn_tower_trace), may be null
+    int solver_edges;     // real edges of the board (E)
+    SolverGeom sg;        // compact geometry of the exact solver, valid when solver_edges <= SOLVER_MAX_EDGES
     std::string err;
 };
 
@@ -142,6 +145,41 @@ static int launch_stem_mma(dbaz_engine* e, const dbaz_state* leaves, const T* w4
     return launch_stem_mma_nt<T, 8>(e, leaves, w48, out, n, cout, st, pl);
 }
 
+// The solver's compact geometry from the engine's action table: edge j = j-th real action, box masks re-indexed
+// from actions to compact edges.
+static cudaError_t build_solver_geom(dbaz_engine* e) {
+    const Board& b = e->board;
+    e->solver_edges = __builtin_popcountll(b.real[0]) + __builtin_popcountll(b.real[1]);
+    std::memset(&e->sg, 0, sizeof e->sg);
+    if (e->solver_edges > SOLVER_MAX_EDGES) return cudaSuccess;
+    std::vector<uint4> tab((size_t)b.A * 2);
+    cudaError_t st = cudaMemcpy(tab.data(), e->ta.act_tab, tab.size() * sizeof(uint4), cudaMemcpyDeviceToHost);
+    if (st != cudaSuccess) return st;
+    SolverGeom& g = e->sg;
+    g.E = e->solver_edges; g.LC = b.nboxes;
+    // every supported board has A <= 44 actions: all real edges live in word 0
+    auto compact = [&](uint64_t lo) {
+        uint32_t m = 0;
+        for (int a = 0; a < 64; ++a)
+            if ((lo >> a) & 1ull) m |= 1u << __builtin_popcountll(b.real[0] & ((1ull << a) - 1ull));
+        return m;
+    };
+    for (int a = 0, j = 0; a < b.A; ++a) {
+        if (!((b.real[0] >> a) & 1ull)) continue;
+        g.act[j] = (uint8_t)a;
+        for (int k = 0; k < 2; ++k) {
+            const uint4 q = tab[2 * a + k];
+            const uint32_t m = compact((uint64_t)q.x | ((uint64_t)q.y << 32));
+            g.ebox[j][k] = m;
+            bool known = m == 0;
+            for (int i = 0; i < g.nboxes && !known; ++i) known = g.box[i] == m;
+            if (!known) g.box[g.nboxes++] = m;
+        }
+        ++j;
+    }
+    return cudaSuccess;
+}
+
 extern "C" {
 
 int dbaz_abi_version(void) { return DBAZ_ABI_VERSION; }
@@ -245,6 +283,7 @@ int dbaz_engine_create(const dbaz_config* cfg, dbaz_engine** out) {
     // an all-empty-board root set so that the engine is usable right after create
     k_reset_roots<<<blocks_for(ta.n_trees, 128), 128>>>(b, ta, nullptr);
     if ((st = cudaDeviceSynchronize()) != cudaSuccess) { cuda_fail(nullptr, "k_reset_roots", st); dbaz_engine_destroy(e); return 1; }
+    if ((st = build_solver_geom(e)) != cudaSuccess) { cuda_fail(nullptr, "solver geometry", st); dbaz_engine_destroy(e); return 1; }
     *out = e;
     return 0;
 }
@@ -812,6 +851,84 @@ int dbaz_search_status(dbaz_engine* e, int64_t* out8, uint64_t stream) {
         return fail(e, buf);
     }
     return 0;
+}
+
+/* ---------------------------------------------------------------- exact solver */
+
+static int solver_unsupported(dbaz_engine* e, const char* fn) {
+    if (e->solver_edges <= SOLVER_MAX_EDGES) return 0;
+    char buf[256];
+    std::snprintf(buf, sizeof buf,
+                  "%s: a %dx%d board has %d edges; the solver supports boards of at most %d edges (1x1..1x10, 2x2..2x6, 3x3, 3x4 "
+                  "and their transposes)", fn, e->board.L, e->board.C, e->solver_edges, SOLVER_MAX_EDGES);
+    return fail(e, buf);
+}
+
+int dbaz_solver_solve(dbaz_engine* e, int8_t* table, int64_t table_bytes, uint64_t stream) {
+    if (!e) return 1;
+    if (solver_unsupported(e, "dbaz_solver_solve")) return 1;
+    const SolverGeom& g = e->sg;
+    const int64_t bytes = (int64_t)1 << g.E;
+    if (!table || table_bytes != bytes) {
+        char buf[160];
+        std::snprintf(buf, sizeof buf, "dbaz_solver_solve: the table of a %d-edge board is 2^%d = %lld bytes, got %lld", g.E, g.E,
+                      (long long)bytes, (long long)table_bytes);
+        return fail(e, buf);
+    }
+    DeviceGuard guard(e->cfg.device);
+    const cudaStream_t st = S(stream);
+    // every entry starts as the sentinel, the full board as 0 (layer E); the layers then write each entry exactly once
+    DBAZ_CK(e, cudaMemsetAsync(table, 0x80, (size_t)bytes, st));
+    DBAZ_CK(e, cudaMemsetAsync(table + (bytes - 1), 0, 1, st));
+    for (int k = g.E - 1; k >= 0; --k) {
+        const uint32_t count = c_binom_host(g.E, k);
+        k_solver_layer<<<blocks_for(count, 256), 256, 0, st>>>(g, table, k, count);
+        if (launch_ok(e, "k_solver_layer")) return 1;
+    }
+    // one reduction over the whole table proves that every entry was written
+    unsigned long long* d_left = nullptr;
+    DBAZ_CK(e, cudaMalloc(&d_left, sizeof(unsigned long long)));
+    unsigned long long left = 0;
+    cudaError_t cst = cudaMemsetAsync(d_left, 0, sizeof(unsigned long long), st);
+    if (cst == cudaSuccess) {
+        const int64_t n16 = bytes / 16;
+        k_solver_check<<<(int)std::min<int64_t>(blocks_for(n16, 256), (int64_t)e->n_sms * 8), 256, 0, st>>>(
+            reinterpret_cast<const uint4*>(table), n16, d_left);
+        cst = cudaGetLastError();
+    }
+    if (cst == cudaSuccess) cst = cudaMemcpyAsync(&left, d_left, sizeof left, cudaMemcpyDeviceToHost, st);
+    if (cst == cudaSuccess) cst = cudaStreamSynchronize(st);
+    cudaFree(d_left);
+    if (cst != cudaSuccess) return cuda_fail(e, "dbaz_solver_solve (table check)", cst);
+    if (left) {
+        char buf[128];
+        std::snprintf(buf, sizeof buf, "dbaz_solver_solve: %llu table entries were never written", left);
+        return fail(e, buf);
+    }
+    return 0;
+}
+
+int dbaz_solver_moves(dbaz_engine* e, const int8_t* table, const dbaz_state* states, int8_t* move_margin, int8_t* margin, int64_t n,
+                      uint64_t stream) {
+    if (!e) return 1;
+    if (solver_unsupported(e, "dbaz_solver_moves")) return 1;
+    if (!table || !states || !move_margin || !margin) return fail(e, "dbaz_solver_moves: null buffer");
+    if (n <= 0) return 0;
+    DeviceGuard guard(e->cfg.device);
+    k_solver_moves<<<blocks_for(n * 32, 256), 256, 0, S(stream)>>>(e->board, e->sg, table, states, move_margin, margin, n);
+    return launch_ok(e, "k_solver_moves");
+}
+
+int dbaz_solver_eval(dbaz_engine* e, const int8_t* table, const dbaz_state* leaf_states, float* priors, float* values, int32_t mode,
+                     int64_t n, uint64_t stream) {
+    if (!e) return 1;
+    if (solver_unsupported(e, "dbaz_solver_eval")) return 1;
+    if (!table || !leaf_states || !priors || !values) return fail(e, "dbaz_solver_eval: null buffer");
+    if (mode < 0 || mode > 1) return fail(e, "dbaz_solver_eval: mode must be 0 (outcome) or 1 (margin)");
+    if (n <= 0) return 0;
+    DeviceGuard guard(e->cfg.device);
+    k_solver_eval<<<blocks_for(n * 32, 256), 256, 0, S(stream)>>>(e->board, e->sg, table, leaf_states, priors, values, mode, n);
+    return launch_ok(e, "k_solver_eval");
 }
 
 }  // extern "C"

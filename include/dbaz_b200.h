@@ -316,6 +316,25 @@ int dbaz_nn_tower_trace(dbaz_engine *e, int64_t *timeline);
 int dbaz_fake_nn(dbaz_engine *e, const dbaz_state *leaf_states, float *priors, float *values, int32_t kind,
                  int64_t n, uint64_t stream);
 
+/* ---- exact solver for boards of at most 32 real edges (dotsboxesaz_b200/csrc/dbaz_solver.cuh, DESIGN.md §10) ----
+ * E = 2LC + L + C real edges; compact edge j = the j-th real action in increasing order; M = played edges as a 32-bit
+ * compact mask.  table: caller-owned int8[2^E], entry M = v(M), the largest net number of boxes the player to move can
+ * still gain against best play (full-game recurrence, no early stop).  The mover's lead d = LC - btc2[to_play] - closed
+ * boxes; final margin = d + v(M), outcome = sign(final margin), both seen by the player to move.  Every entry point rejects
+ * boards with E > 32 (4x4 and up) with an error message.
+ * dbaz_solver_solve: fills the table (one kernel per popcount layer) and checks that every entry was written;
+ * table_bytes must be 2^E.  Synchronises `stream`. */
+int dbaz_solver_solve(dbaz_engine *e, int8_t *table, int64_t table_bytes, uint64_t stream);
+/* move_margin int8[n][A]: d + (c > 0 ? c + v(M|a) : -v(M|a)) for every free edge a (c = boxes a closes), -128 for
+ * played edges and padding; margin int8[n]: the final margin. */
+int dbaz_solver_moves(dbaz_engine *e, const int8_t *table, const dbaz_state *states, int8_t *move_margin, int8_t *margin,
+                      int64_t n, uint64_t stream);
+/* A perfect-play evaluator for dbaz_search_step's leaves: priors float32[n][A] = 1/k (k = __fdiv_rn(1, k)) on the k moves
+ * whose margin has the sign of the outcome, 0 elsewhere; values float32[n] = outcome (mode 0) or final margin / (L C)
+ * (mode 1).  A function of the eval-cache key; no allocation and no synchronisation (capturable in a CUDA graph). */
+int dbaz_solver_eval(dbaz_engine *e, const int8_t *table, const dbaz_state *leaf_states, float *priors, float *values,
+                     int32_t mode, int64_t n, uint64_t stream);
+
 #ifdef __cplusplus
 }
 #endif
