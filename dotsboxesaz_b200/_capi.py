@@ -86,6 +86,8 @@ SYMBOLS = {
     "dbaz_solver_solve": (C.c_int, [_P, _P, _I64, _U64]),
     "dbaz_solver_moves": (C.c_int, [_P, _P, _P, _P, _P, _I64, _U64]),
     "dbaz_solver_eval": (C.c_int, [_P, _P, _P, _P, _P, _I32, _I64, _U64]),
+    "dbaz_endgame_moves": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _U64]),
+    "dbaz_endgame_eval": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _I64, _U64]),
 }
 
 _lib = None

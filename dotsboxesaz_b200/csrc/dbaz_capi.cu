@@ -16,6 +16,7 @@
 #include "dbaz_tower.cuh"
 #include "dbaz_loop.cuh"
 #include "dbaz_solver.cuh"
+#include "dbaz_endgame.cuh"
 
 using namespace dbaz;
 
@@ -38,6 +39,8 @@ struct dbaz_engine {
     long long* tower_dbg; // caller-owned timeline buffer (dbaz_nn_tower_trace), may be null
     int solver_edges;     // real edges of the board (E)
     SolverGeom sg;        // compact geometry of the exact solver, valid when solver_edges <= SOLVER_MAX_EDGES
+    uint16_t* eg_order;   // endgame_order_host: the masks of every f <= 16 by popcount (ENDGAME_ORDER_ENTRIES)
+    int eg_blocks[2][ENDGAME_MAX_FREE + 1];  // resident CTAs per SM of k_endgame_moves / k_endgame_eval by max_free
     std::string err;
 };
 
@@ -180,6 +183,25 @@ static cudaError_t build_solver_geom(dbaz_engine* e) {
     return cudaSuccess;
 }
 
+// The endgame solver's mask order, and its kernels' shared-memory opt-in and occupancy for every max_free (set once
+// here: never during a stream capture).
+static cudaError_t build_endgame(dbaz_engine* e) {
+    std::vector<uint16_t> order(ENDGAME_ORDER_ENTRIES);
+    endgame_order_host(order.data());
+    cudaError_t st = cudaMalloc(&e->eg_order, order.size() * sizeof(uint16_t));
+    if (st == cudaSuccess) st = cudaMemcpy(e->eg_order, order.data(), order.size() * sizeof(uint16_t), cudaMemcpyHostToDevice);
+    const void* kernels[2] = {(const void*)k_endgame_moves, (const void*)k_endgame_eval};
+    for (int k = 0; k < 2 && st == cudaSuccess; ++k) {
+        st = cudaFuncSetAttribute(kernels[k], cudaFuncAttributeMaxDynamicSharedMemorySize, endgame_smem_bytes(ENDGAME_MAX_FREE));
+        for (int f = 0; f <= ENDGAME_MAX_FREE && st == cudaSuccess; ++f) {
+            int nb = 0;
+            st = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernels[k], ENDGAME_THREADS, endgame_smem_bytes(f));
+            e->eg_blocks[k][f] = std::max(1, nb);
+        }
+    }
+    return st;
+}
+
 extern "C" {
 
 int dbaz_abi_version(void) { return DBAZ_ABI_VERSION; }
@@ -284,6 +306,7 @@ int dbaz_engine_create(const dbaz_config* cfg, dbaz_engine** out) {
     k_reset_roots<<<blocks_for(ta.n_trees, 128), 128>>>(b, ta, nullptr);
     if ((st = cudaDeviceSynchronize()) != cudaSuccess) { cuda_fail(nullptr, "k_reset_roots", st); dbaz_engine_destroy(e); return 1; }
     if ((st = build_solver_geom(e)) != cudaSuccess) { cuda_fail(nullptr, "solver geometry", st); dbaz_engine_destroy(e); return 1; }
+    if ((st = build_endgame(e)) != cudaSuccess) { cuda_fail(nullptr, "endgame solver set-up", st); dbaz_engine_destroy(e); return 1; }
     *out = e;
     return 0;
 }
@@ -304,6 +327,7 @@ void dbaz_engine_destroy(dbaz_engine* e) {
     cudaFree(e->d_status);
     cudaFree(e->d_tower_err);
     cudaFree(e->d_cache_epoch);
+    cudaFree(e->eg_order);
     delete e;
 }
 
@@ -929,6 +953,45 @@ int dbaz_solver_eval(dbaz_engine* e, const int8_t* table, const dbaz_state* leaf
     DeviceGuard guard(e->cfg.device);
     k_solver_eval<<<blocks_for(n * 32, 256), 256, 0, S(stream)>>>(e->board, e->sg, table, leaf_states, priors, values, mode, n);
     return launch_ok(e, "k_solver_eval");
+}
+
+/* ---------------------------------------------------------------- exact endgame solver */
+
+static int endgame_bad_max_free(dbaz_engine* e, const char* fn, int max_free) {
+    if (max_free >= 0 && max_free <= ENDGAME_MAX_FREE) return 0;
+    char buf[160];
+    std::snprintf(buf, sizeof buf, "%s: max_free must be in [0, %d], got %d", fn, ENDGAME_MAX_FREE, max_free);
+    return fail(e, buf);
+}
+
+// persistent grid: at most the CTAs resident at once, at most one per row
+static int endgame_grid(const dbaz_engine* e, int kernel, int max_free, int64_t n) {
+    return (int)std::min<int64_t>(n, (int64_t)e->n_sms * e->eg_blocks[kernel][max_free]);
+}
+
+int dbaz_endgame_moves(dbaz_engine* e, const dbaz_state* states, int8_t* move_margin, int8_t* margin, int32_t max_free, int64_t n,
+                       uint64_t stream) {
+    if (!e) return 1;
+    if (endgame_bad_max_free(e, "dbaz_endgame_moves", max_free)) return 1;
+    if (!states || !move_margin || !margin) return fail(e, "dbaz_endgame_moves: null buffer");
+    if (n <= 0) return 0;
+    DeviceGuard guard(e->cfg.device);
+    k_endgame_moves<<<endgame_grid(e, 0, max_free, n), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
+        e->board, e->ta.act_tab, e->eg_order, states, EndgameMovesOut{move_margin, margin}, max_free, n);
+    return launch_ok(e, "k_endgame_moves");
+}
+
+int dbaz_endgame_eval(dbaz_engine* e, const dbaz_state* leaf_states, float* priors, float* values, int32_t mode, int32_t keep_priors,
+                      int32_t max_free, int64_t n, uint64_t stream) {
+    if (!e) return 1;
+    if (endgame_bad_max_free(e, "dbaz_endgame_eval", max_free)) return 1;
+    if (!leaf_states || !priors || !values) return fail(e, "dbaz_endgame_eval: null buffer");
+    if (mode < 0 || mode > 1) return fail(e, "dbaz_endgame_eval: mode must be 0 (outcome) or 1 (margin)");
+    if (n <= 0) return 0;
+    DeviceGuard guard(e->cfg.device);
+    k_endgame_eval<<<endgame_grid(e, 1, max_free, n), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
+        e->board, e->ta.act_tab, e->eg_order, leaf_states, EndgameEvalOut{priors, values, mode, keep_priors ? 1 : 0}, max_free, n);
+    return launch_ok(e, "k_endgame_eval");
 }
 
 }  // extern "C"

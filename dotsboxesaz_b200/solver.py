@@ -151,14 +151,21 @@ def grade(solver, states, policy=None, value=None, z=None):
     value_outcome_accuracy  share of rows where value > 1/3 (win), < -1/3 (loss) or else (draw) matches the outcome
     value_mse               mean squared error of value against the outcome
     z_agreement             share of rows whose sign(z) equals the outcome
-    Only the figures whose inputs are given are returned, plus n."""
+    Only the figures whose inputs are given are returned, plus n.
+    With an endgame.EndgameSolver the means run over the solvable rows only, and n_solved counts them."""
     mm, mg = solver.moves(states)
     dev = mm.device
+    out = {"n": int(mm.shape[0])}
+    keep = None
+    if hasattr(solver, "max_free"):  # an EndgameSolver: unsolvable rows read ILLEGAL and are dropped
+        keep = mg != ILLEGAL
+        mm, mg = mm[keep], mg[keep]
+        out["n_solved"] = int(mm.shape[0])
     o = torch.sign(mg).to(torch.float64)
     opt = (mm != ILLEGAL) & (torch.sign(mm) == torch.sign(mg).unsqueeze(1))
-    out = {"n": int(mm.shape[0])}
     if policy is not None:
-        p = torch.as_tensor(policy).to(device=dev, dtype=torch.float64).reshape(mm.shape)
+        p = torch.as_tensor(policy).to(device=dev, dtype=torch.float64)
+        p = (p.reshape(-1, solver.A)[keep] if keep is not None else p).reshape(mm.shape)
         best = p.max(1, keepdim=True).values
         ar = torch.arange(solver.A, device=dev)
         first = torch.where(p == best, ar, solver.A).min(1).values
@@ -166,17 +173,20 @@ def grade(solver, states, policy=None, value=None, z=None):
         out["optimal_mass"] = (p * opt).sum(1).mean().item()
     if value is not None:
         v = torch.as_tensor(value).to(device=dev, dtype=torch.float64).reshape(-1)
+        v = v[keep] if keep is not None else v
         pred = torch.where(v > 1.0 / 3.0, 1.0, torch.where(v < -1.0 / 3.0, -1.0, 0.0))
         out["value_outcome_accuracy"] = (pred == o).double().mean().item()
         out["value_mse"] = ((v - o) ** 2).mean().item()
     if z is not None:
         zz = torch.as_tensor(z).to(device=dev, dtype=torch.float64).reshape(-1)
+        zz = zz[keep] if keep is not None else zz
         out["z_agreement"] = (torch.sign(zz) == o).double().mean().item()
     return out
 
 
 def grade_samples(solver, batch):
-    """grade() of a samples.SampleBatch: its positions rebuilt from the feature planes, pi as the policy, and z."""
+    """grade() of a samples.SampleBatch: its positions rebuilt from the feature planes, pi as the policy, and z.  `solver`
+    is a Solver or an endgame.EndgameSolver."""
     return grade(solver, solver.states_from_planes(batch.planes), policy=batch.pi, z=batch.z)
 
 

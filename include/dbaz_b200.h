@@ -335,6 +335,21 @@ int dbaz_solver_moves(dbaz_engine *e, const int8_t *table, const dbaz_state *sta
 int dbaz_solver_eval(dbaz_engine *e, const int8_t *table, const dbaz_state *leaf_states, float *priors, float *values,
                      int32_t mode, int64_t n, uint64_t stream);
 
+/* ---- exact endgame solver for every board (dotsboxesaz_b200/csrc/dbaz_endgame.cuh, DESIGN.md §11) ----
+ * A state with f free real edges is solvable when f <= max_free; max_free must be in [0, 16].  Its value v(M) (as above)
+ * comes from a retrograde over the 2^f subsets of its free edges, in shared memory, so no table is needed and every
+ * board the engine plays is supported.  Margins, outcomes and move margins are those of the solver entries above.
+ * Neither entry allocates or synchronises (both are capturable in a CUDA graph).
+ * dbaz_endgame_moves: move_margin int8[n][A] and margin int8[n] as dbaz_solver_moves for solvable states; every byte of
+ * an unsolvable state's row and its margin is -128. */
+int dbaz_endgame_moves(dbaz_engine *e, const dbaz_state *states, int8_t *move_margin, int8_t *margin, int32_t max_free,
+                       int64_t n, uint64_t stream);
+/* An endgame-exact evaluator, run after another evaluator on the same leaves: it rewrites only the rows of solvable
+ * leaves, with priors as dbaz_solver_eval (left as they are when keep_priors != 0) and values = outcome (mode 0) or final
+ * margin / (L C) (mode 1).  Every other row keeps its bits.  A function of the eval-cache key. */
+int dbaz_endgame_eval(dbaz_engine *e, const dbaz_state *leaf_states, float *priors, float *values, int32_t mode,
+                      int32_t keep_priors, int32_t max_free, int64_t n, uint64_t stream);
+
 #ifdef __cplusplus
 }
 #endif
