@@ -40,7 +40,7 @@ struct dbaz_engine {
     int solver_edges;     // real edges of the board (E)
     SolverGeom sg;        // compact geometry of the exact solver, valid when solver_edges <= SOLVER_MAX_EDGES
     uint16_t* eg_order;   // endgame_order_host: the masks of every f <= 16 by popcount (ENDGAME_ORDER_ENTRIES)
-    int eg_blocks[2][ENDGAME_MAX_FREE + 1];  // resident CTAs per SM of k_endgame_moves / k_endgame_eval by max_free
+    int eg_blocks[3][ENDGAME_MAX_FREE + 1];  // resident CTAs per SM of k_endgame_moves / k_endgame_eval / k_selfplay_adjudicate by max_free
     std::string err;
 };
 
@@ -190,8 +190,8 @@ static cudaError_t build_endgame(dbaz_engine* e) {
     endgame_order_host(order.data());
     cudaError_t st = cudaMalloc(&e->eg_order, order.size() * sizeof(uint16_t));
     if (st == cudaSuccess) st = cudaMemcpy(e->eg_order, order.data(), order.size() * sizeof(uint16_t), cudaMemcpyHostToDevice);
-    const void* kernels[2] = {(const void*)k_endgame_moves, (const void*)k_endgame_eval};
-    for (int k = 0; k < 2 && st == cudaSuccess; ++k) {
+    const void* kernels[3] = {(const void*)k_endgame_moves, (const void*)k_endgame_eval, (const void*)k_selfplay_adjudicate};
+    for (int k = 0; k < 3 && st == cudaSuccess; ++k) {
         st = cudaFuncSetAttribute(kernels[k], cudaFuncAttributeMaxDynamicSharedMemorySize, endgame_smem_bytes(ENDGAME_MAX_FREE));
         for (int f = 0; f <= ENDGAME_MAX_FREE && st == cudaSuccess; ++f) {
             int nb = 0;
@@ -992,6 +992,19 @@ int dbaz_endgame_eval(dbaz_engine* e, const dbaz_state* leaf_states, float* prio
     k_endgame_eval<<<endgame_grid(e, 1, max_free, n), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
         e->board, e->ta.act_tab, e->eg_order, leaf_states, EndgameEvalOut{priors, values, mode, keep_priors ? 1 : 0}, max_free, n);
     return launch_ok(e, "k_endgame_eval");
+}
+
+int dbaz_selfplay_adjudicate(dbaz_engine* e, const dbaz_selfplay_buffers* bufs, int8_t* margin, int32_t max_free, int32_t first,
+                             uint64_t stream) {
+    if (!e || !bufs) return 1;
+    if (endgame_bad_max_free(e, "dbaz_selfplay_adjudicate", max_free)) return 1;
+    if (!margin) return fail(e, "dbaz_selfplay_adjudicate: null margin");
+    SelfplayArgs sp;
+    if (int rc = selfplay_args(e, bufs, sp)) return rc;
+    DeviceGuard guard(e->cfg.device);
+    k_selfplay_adjudicate<<<endgame_grid(e, 2, max_free, e->ta.n_trees), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
+        e->board, e->ta, e->eg_order, sp, margin, max_free, first ? 1 : 0);
+    return launch_ok(e, "k_selfplay_adjudicate");
 }
 
 }  // extern "C"

@@ -17,6 +17,8 @@
 //   11 <= f <= 16      the whole CTA per position, a 2^f-byte table, __syncthreads between popcount layers.
 // Layer k of an f-edge table is the k-subsets of f bits in increasing order, read from a table of every such ordering
 // (endgame_order_host, uploaded once per engine), so a thread reads its mask instead of unranking it.
+// Where the rows come from is a template parameter (Rows): a contiguous state array here (StateRows), the roots of the
+// self-play trees in dbaz_selfplay.cuh.  A row the source does not qualify is classified unsolvable without being read.
 #pragma once
 #include "dbaz_solver.cuh"
 
@@ -197,9 +199,16 @@ struct EndgameEvalOut {
     }
 };
 
-template <class Out>
+// Row source of k_endgame_moves / k_endgame_eval: state w of a contiguous array, every row qualifies.
+struct StateRows {
+    const dbaz_state* __restrict__ states;
+    __device__ __forceinline__ bool qualifies(int64_t) const { return true; }
+    __device__ __forceinline__ dbaz_state state(int64_t w) const { return states[w]; }
+};
+
+template <class Rows, class Out>
 __device__ __forceinline__ void endgame_rows(const Board& b, const uint4* __restrict__ act_tab, const uint16_t* __restrict__ order,
-                                             const dbaz_state* __restrict__ states, const Out& out, int max_free, int64_t n) {
+                                             const Rows& rows, const Out& out, int max_free, int64_t n) {
     extern __shared__ __align__(16) int8_t eg_table[];  // endgame_smem_bytes(max_free)
     __shared__ uint32_t geo[ENDGAME_WARPS][ENDGAME_MAX_FREE];
     __shared__ uint16_t list[3][ENDGAME_THREADS];  // rows of this pass for the warp tier, the CTA tier, unsolvable
@@ -213,7 +222,7 @@ __device__ __forceinline__ void endgame_rows(const Board& b, const uint4* __rest
         __syncthreads();
         const int64_t w = first + stride * tid;
         if (w < n) {
-            const int f = endgame_f(b, states[w]);
+            const int f = rows.qualifies(w) ? endgame_f(b, rows.state(w)) : ENDGAME_MAX_FREE + 1;
             const int tier = f <= warp_max ? 0 : f <= max_free ? 1 : 2;
             list[tier][atomicAdd(&count[tier], 1)] = (uint16_t)tid;
         }
@@ -223,7 +232,7 @@ __device__ __forceinline__ void endgame_rows(const Board& b, const uint4* __rest
         int8_t* Tw = eg_table + (warp << ENDGAME_WARP_MAX_FREE);
         for (int j = warp; j < count[0]; j += ENDGAME_WARPS) {
             const int64_t row = first + stride * list[0][j];
-            const dbaz_state s = states[row];
+            const dbaz_state s = rows.state(row);
             const EndgameRow p = endgame_row(b, act_tab, s, geo[warp], lane);
             __syncwarp();
             endgame_table<32>(Tw, geo[warp], p.f, lane, order);
@@ -235,7 +244,7 @@ __device__ __forceinline__ void endgame_rows(const Board& b, const uint4* __rest
             const int64_t row = first + stride * list[1][j];
             EndgameRow p;
             if (warp == 0) {
-                const dbaz_state s = states[row];
+                const dbaz_state s = rows.state(row);
                 p = endgame_row(b, act_tab, s, geo[0], lane);
                 if (lane == 0) cta_f = p.f;
             }
@@ -251,13 +260,13 @@ __device__ __forceinline__ void endgame_rows(const Board& b, const uint4* __rest
 __global__ void __launch_bounds__(ENDGAME_THREADS, 3) k_endgame_moves(Board b, const uint4* __restrict__ act_tab,
                                                                   const uint16_t* __restrict__ order, const dbaz_state* __restrict__ states,
                                                                   EndgameMovesOut out, int max_free, int64_t n) {
-    endgame_rows(b, act_tab, order, states, out, max_free, n);
+    endgame_rows(b, act_tab, order, StateRows{states}, out, max_free, n);
 }
 
 __global__ void __launch_bounds__(ENDGAME_THREADS, 3) k_endgame_eval(Board b, const uint4* __restrict__ act_tab,
                                                                  const uint16_t* __restrict__ order, const dbaz_state* __restrict__ leaves,
                                                                  EndgameEvalOut out, int max_free, int64_t n) {
-    endgame_rows(b, act_tab, order, leaves, out, max_free, n);
+    endgame_rows(b, act_tab, order, StateRows{leaves}, out, max_free, n);
 }
 
 }  // namespace dbaz

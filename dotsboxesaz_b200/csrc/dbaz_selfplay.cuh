@@ -10,8 +10,12 @@
 //   k_selfplay_restart  after the re-root: games that go on get the simulation budget of their number of legal moves
 //                       (n_searches) and their row of Dirichlet noise times the legal mask (mcts.py:220-223); the others
 //                       are told to leave their tree alone (num_reads = -3, k_search_begin); counts the games still on.
+//   k_selfplay_adjudicate  optional, after the restart: a game whose new root has f <= max_free free edges ends there
+//                       with the exact final margin of that root (the endgame solver of dbaz_endgame.cuh); its root is
+//                       not searched and gives no sample.
 #pragma once
 #include "dbaz_tree_kernels.cuh"
+#include "dbaz_endgame.cuh"
 
 namespace dbaz {
 
@@ -149,6 +153,43 @@ __global__ void __launch_bounds__(SP_WARPS * 32) k_selfplay_restart(Board b, Tre
         sp.reads[t] = go_on ? sp.reads_by_k[k] : -3;
         if (go_on) atomicAdd(sp.left, 1);
     }
+}
+
+// Row source of k_selfplay_adjudicate: row t is the root of tree t (node 0 of its pool).  Only trees that restarted at
+// this check (first, or a move was drawn) and go on qualify; any other tree is not read.
+struct RootRows {
+    TreeArgs ta;
+    const int8_t* searching;
+    const int32_t* moves;
+    int first;
+    __device__ __forceinline__ bool qualifies(int64_t t) const { return (first || moves[t] >= 0) && searching[t] == 1; }
+    __device__ __forceinline__ dbaz_state state(int64_t t) const { return load_hdr(node_ptr(ta, (int)t, 0)); }
+};
+
+// A solvable qualifying root ends its game: its final margin goes to margin[t], the tree stops searching, k_search_begin
+// leaves it alone and it no longer counts as a game going on.  Every other tree is left as it is.
+struct AdjudicateOut {
+    int8_t* margin;
+    int8_t* searching;
+    int32_t* reads;
+    int32_t* left;
+    static constexpr bool kUnsolvable = false;
+    __device__ __forceinline__ void unsolvable(const Board&, int64_t, int) const {}
+    __device__ __forceinline__ void solved(const Board&, const EndgameRow& p, const int8_t* T, const uint32_t*, int64_t t,
+                                           int lane) const {
+        if (lane == 0) {
+            margin[t] = (int8_t)(p.d + T[0]);
+            searching[t] = 0;
+            reads[t] = -3;
+            atomicSub(left, 1);
+        }
+    }
+};
+
+__global__ void __launch_bounds__(ENDGAME_THREADS, 3) k_selfplay_adjudicate(Board b, TreeArgs ta, const uint16_t* __restrict__ order,
+                                                                        SelfplayArgs sp, int8_t* margin, int max_free, int first) {
+    endgame_rows(b, ta.act_tab, order, RootRows{ta, sp.searching, sp.moves, first},
+                 AdjudicateOut{margin, sp.searching, sp.reads, sp.left}, max_free, (int64_t)ta.n_trees);
 }
 
 }  // namespace dbaz

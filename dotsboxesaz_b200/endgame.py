@@ -10,6 +10,8 @@ EndgameEvaluator  wraps any evaluator: exact priors and values on the leaves tha
                   output on every other leaf.
 solver.grade / solver.grade_samples take an EndgameSolver too and grade the solvable rows.
 """
+import ctypes as C
+
 import torch
 
 from ._capi import RESULT_NONE
@@ -94,6 +96,19 @@ class EndgameSolver:
         n = leaf_states.shape[0]
         eng._ck(eng.lib.dbaz_endgame_eval(eng._h, _ptr(leaf_states), _ptr(priors), _ptr(values), int(mode), 1 if keep_priors else 0,
                                           self.max_free, n, eng._stream()))
+
+    def adjudicate(self, bufs, margin, first=False):
+        """dbaz_selfplay_adjudicate, after Engine.selfplay_restart(bufs, first): every game of the asynchronous self-play
+        loop whose new root has at most max_free free edges ends there, with the root's final margin in margin (int8
+        [n_games], ILLEGAL elsewhere)."""
+        eng = self.eng
+        eng._ck(eng.lib.dbaz_selfplay_adjudicate(eng._h, C.byref(bufs), _ptr(margin), self.max_free, 1 if first else 0, eng._stream()))
+
+    def full_states(self, n):
+        """n states with every real edge played (f = 0)."""
+        st = self.eng.new_states(n)
+        st[:, :2] = self._real
+        return st
 
     def states_from_planes(self, planes):
         """Packed states [n, 4] from feature rows (get_features().ravel(), int16 or uint8 as in SampleBatch.planes), on

@@ -38,6 +38,18 @@ def _n_searches(n_valid, num_read):
     return min(4 * math.factorial(n_valid), num_read)  # self_play.py:64-65
 
 
+def _game_outcomes(final, result, margin):
+    """Per game (int8 tensors [n]): the player whose sample rows get z = +outcome, and the outcome; every other row of
+    the game gets -outcome.  A game played out: just_played of its terminal state and its result.  A game adjudicated
+    at a root (margin != ILLEGAL, the root's final margin): that root's player to move and sign(margin)."""
+    from .solver import ILLEGAL
+    raw = final.view(torch.uint8).reshape(-1, 32)
+    adj = margin != ILLEGAL
+    player = torch.where(adj, raw[:, 20], raw[:, 21]).to(torch.int8)
+    outcome = torch.where(adj, torch.sign(margin), result.to(torch.int8))
+    return player, outcome
+
+
 def _dataset(rows, generation, with_features):
     """The DataFrame of self_play.py:95-156 from row dicts (same columns, dtypes and MultiIndex)."""
     n = len(rows)
@@ -137,9 +149,17 @@ class BatchedSelfPlay:
     evaluator(engine): fills engine.priors / engine.values from engine.planes (dotsboxesaz_b200.nn.DeviceEvaluator
     or engine.FakeNetEvaluator).  seeds: one legacy-MT19937 seed per game; per move the stream yields the
     Dirichlet draw (if alpha > 0) and then the uniform of np.random.choice, the reference's order (SURVEY 8c).
+
+    adjudicate (default: params.self_play.adjudicate; None = off): max_free in 0 .. 16.  A game ends at the first root
+    that is still going on and has at most max_free free edges; that root is not searched and gives no sample, and every
+    row of the game takes its z from perfect play out of it (endgame.EndgameSolver): +outcome for the rows of the root's
+    player to move, -outcome for the others.  So positions with f <= max_free leave the training data.  The natural
+    evaluator to pair it with is EndgameEvaluator(inner, EndgameSolver(engine, m)) with m >= max_free, so that the net
+    is never asked about the positions it no longer trains on (not enforced).  Games that end at a majority earlier are
+    played as without adjudication.
     """
 
-    def __init__(self, engine, evaluator, params, graph_waves=16, pending=None, adaptive=None):
+    def __init__(self, engine, evaluator, params, graph_waves=16, pending=None, adaptive=None, adjudicate=None):
         self.eng = engine
         self.ev = evaluator
         self.params = params
@@ -153,6 +173,13 @@ class BatchedSelfPlay:
         self.played_games = []
         self.rows = []
         self.total_sims = 0
+        m = params.self_play.get("adjudicate", None) if adjudicate is None else adjudicate
+        self.endgame = None
+        if m is not None:
+            from .endgame import EndgameSolver
+            if not 0 <= int(m) <= 16:
+                raise ValueError("adjudicate must be a max_free in 0 .. 16 or None, got %r" % (m,))
+            self.endgame = EndgameSolver(engine, int(m))
 
     def play_games(self, games_idxs, seeds=None, start_states=None, with_features=True):
         eng, sp = self.eng, self.params.self_play
@@ -172,6 +199,7 @@ class BatchedSelfPlay:
         temperature = [None] * n
         hist = [[] for _ in range(n)]  # per game: row dicts of every searched root
         moves_played = [[] for _ in range(n)]
+        margin = np.full(n, -128, dtype=np.int8)  # final margin of the root a game was adjudicated at, -128 (ILLEGAL) if none
         move_i = -1
         while active.any():
             move_i += 1
@@ -181,6 +209,12 @@ class BatchedSelfPlay:
             feats = eng.features(roots, torch.int16).cpu().numpy().reshape(n, -1) if with_features else None
             roots_np = eng.states_to_numpy(roots)
             active &= (res == RESULT_NONE)
+            if self.endgame is not None:
+                due = active & (self.endgame.free_edges(roots).cpu().numpy() <= self.endgame.max_free)
+                if due.any():
+                    idx = np.flatnonzero(due)
+                    margin[idx] = self.endgame.margin(roots[torch.from_numpy(idx).to(roots.device)].contiguous()).cpu().numpy()
+                    active &= ~due
             if not active.any():
                 break
             reads = np.full(n, -1, dtype=np.int32)
@@ -210,11 +244,12 @@ class BatchedSelfPlay:
             eng.advance_roots(moves, reuse=bool(sp.reuse_mcts_tree))
         info = eng.status()
         self.total_sims = info["sims"]
-        final = eng.states_to_numpy(eng.root_states())
-        res = eng.result(eng.root_states()).cpu().numpy()
+        info["adjudicated"] = int((margin[:len(games_idxs)] != -128).sum())
+        final = eng.root_states()
+        winners, outcomes = (x.cpu().numpy() for x in _game_outcomes(final, eng.result(final), torch.from_numpy(margin).to(final.device)))
         for g in range(len(games_idxs)):
-            z = int(res[g])
-            winner = int(final["just_played"][g])
+            z = int(outcomes[g])
+            winner = int(winners[g])
             for r in hist[g]:
                 vs = r["visits"].sum()
                 r["pi"] = r["visits"] / (vs or 1.0)
@@ -251,12 +286,20 @@ class BatchedSelfPlay:
             noise_all = g / g.sum(-1, keepdim=True)
         temperature = None
         hist_states, hist_visits, hist_active, hist_moves, hist_stats, hist_q = [], [], [], [], [], []
+        margin = torch.full((n,), -128, dtype=torch.int8, device=dev)  # final margin of an adjudicated game's root, else ILLEGAL
+        full = self.endgame.full_states(n) if self.endgame is not None else None
         for move_i in range(n_moves):
             if move_i in temp_sched:
                 temperature = float(temp_sched[move_i])
             roots = eng.root_states()
             valid = eng.valid_moves(roots)
             active = eng.result(roots) == RESULT_NONE
+            if self.endgame is not None:
+                # roots reaching f <= max_free now: solved once (the other rows solve the f = 0 full board) and out of play
+                active &= margin == -128
+                due = active & (self.endgame.free_edges(roots) <= self.endgame.max_free)
+                margin = torch.where(due, self.endgame.margin(torch.where(due.unsqueeze(1), roots, full).contiguous()), margin)
+                active &= ~due
             k = n_moves - move_i  # legal moves left: one edge is played per move
             reads = torch.where(active, torch.full((n,), _n_searches(k, num_read), dtype=torch.int32, device=dev),
                                 torch.full((n,), -1, dtype=torch.int32, device=dev))
@@ -278,8 +321,9 @@ class BatchedSelfPlay:
         res = eng.result(final)
         info = eng.status()  # the only host synchronisation of the whole batch of games
         self.total_sims = info["sims"]
+        info["adjudicated"] = int((margin != -128).sum())
         self._device_hist = dict(states=hist_states, visits=hist_visits, active=hist_active, moves=hist_moves, stats=hist_stats,
-                                 q=hist_q, final=final, result=res, games_idxs=games_idxs, with_features=with_features,
+                                 q=hist_q, final=final, result=res, margin=margin, games_idxs=games_idxs, with_features=with_features,
                                  noise=noise_all)  # the pre-drawn Dirichlet samples [move, game, A]: a run can be replayed
         return info
 
@@ -330,6 +374,7 @@ class BatchedSelfPlay:
         searching = torch.ones((n,), dtype=torch.int8, device=dev)
         moves = torch.full((n,), -1, dtype=torch.int32, device=dev)
         left_dev = torch.zeros((1,), dtype=torch.int32, device=dev)
+        margin = torch.full((n,), -128, dtype=torch.int8, device=dev)  # final margin of an adjudicated game's root, else ILLEGAL
         u_all = torch.rand((n_moves, n), dtype=torch.float64, device=dev, generator=gen)  # one uniform per (move, game): the draw of the move
 
         eng.pending = 1
@@ -349,17 +394,23 @@ class BatchedSelfPlay:
                                h_states=ptr(h_states), h_visits=ptr(h_visits), h_active=ptr(h_active), h_moves=ptr(h_moves),
                                h_stats=ptr(h_stats), h_q=ptr(h_q), noise_buf=ptr(noise_buf), reads=ptr(reads), left=ptr(left_dev))
         keep = (bufs, inv_temp, reads_by_k, u_all, noise_all)  # the kernels hold raw pointers: these tensors live until the loop ends
+        adj = self.endgame
 
-        eng.selfplay_restart(bufs, first=True)  # every tree begins its first search
+        eng.selfplay_restart(bufs, first=True)  # every tree begins its first search ...
+        if adj is not None:
+            adj.adjudicate(bufs, margin, first=True)  # ... unless its start state is adjudicated already
         eng.begin(reads, noise_arg, coeff, 1)
 
         def finish():
             """Trees whose search has finished: record the sample, draw the move (k_selfplay_pick), re-root
-            (k_advance_roots), budget and noise of the next search (k_selfplay_restart), begin it (k_search_begin).
-            Four launches on in-place state, captured as one CUDA graph."""
+            (k_advance_roots), budget and noise of the next search (k_selfplay_restart), end the games whose new root is
+            adjudicated (k_selfplay_adjudicate, with adjudication on), begin the other searches (k_search_begin).
+            Four or five launches on in-place state, captured as one CUDA graph."""
             eng.selfplay_pick(bufs)
             eng.advance_roots(moves, reuse=bool(sp.reuse_mcts_tree))
             eng.selfplay_restart(bufs)
+            if adj is not None:
+                adj.adjudicate(bufs, margin)
             eng.begin(reads, noise_arg, coeff, 1)
 
         # capture_begin / capture_end directly: the torch.cuda.graph() context empties the caching allocator (and the pinned
@@ -408,9 +459,11 @@ class BatchedSelfPlay:
         res = eng.result(final)
         info = eng.status()
         self.total_sims = info["sims"]
+        info["adjudicated"] = int((margin != -128).sum())
+        info["checks"] = i  # finish-graph replays of the batch
         self._device_hist = dict(states=list(h_states.unbind(0)), visits=list(h_visits.unbind(0)), active=list(h_active.unbind(0)),
                                  moves=list(h_moves.unbind(0)), stats=list(h_stats.unbind(0)), q=list(h_q.unbind(0)), final=final,
-                                 result=res, games_idxs=games_idxs, with_features=with_features,
+                                 result=res, margin=margin, games_idxs=games_idxs, with_features=with_features,
                                  noise=noise_all if alpha > 0 else None,  # pre-drawn Dirichlet samples [move, game, A]
                                  uniforms=u_all, inv_temp=inv_temp)              # ... and what drew the moves
         del keep
@@ -433,9 +486,9 @@ class BatchedSelfPlay:
         pi = v / v.sum(1, keepdim=True).clamp_min(1.0)
         slot, mi = idx % n, idx // n
         to_play = sel.view(torch.uint8).reshape(-1, 32)[:, 20].to(torch.int8)
-        winner = (h["final"].view(torch.uint8).reshape(n, 32)[:, 21]).to(torch.int8)[slot]  # just_played of the terminal state
-        z_final = h["result"].float()[slot]
-        z = torch.where(to_play == winner, z_final, -z_final)
+        winner, outcome = _game_outcomes(h["final"], h["result"], h["margin"])
+        z_final = outcome.float()[slot]
+        z = torch.where(to_play == winner[slot], z_final, -z_final)
         return planes, pi, z, slot, mi
 
     def get_games_moves(self):
@@ -473,8 +526,8 @@ class BatchedSelfPlay:
         move = pick(prev).astype(np.int16)
         g_of = torch.arange(n, device=act.device).unsqueeze(1).expand(n, M).reshape(-1)[sel].cpu().numpy()
         m_of = torch.arange(M, device=act.device).unsqueeze(0).expand(n, M).reshape(-1)[sel].cpu().numpy()
-        res = h["result"].cpu().numpy().astype(np.int64)
-        winner = eng.states_to_numpy(h["final"])["just_played"]
+        winner, res = (x.cpu().numpy() for x in _game_outcomes(h["final"], h["result"], h["margin"]))
+        res = res.astype(np.int64)
         z = np.where(player == winner[g_of], res[g_of], -res[g_of])
         games = np.asarray(h["games_idxs"])
         if isinstance(generation, (list, tuple)):
@@ -502,8 +555,7 @@ class BatchedSelfPlay:
         """Turn the device-resident history of play_games_device() into the row dicts of get_datasets()."""
         h, eng = self._device_hist, self.eng
         n = eng.n_games
-        res = h["result"].cpu().numpy()
-        winner = eng.states_to_numpy(h["final"])["just_played"]
+        winner, res = (x.cpu().numpy() for x in _game_outcomes(h["final"], h["result"], h["margin"]))
         act = torch.stack(h["active"]).cpu().numpy()
         moves = torch.stack(h["moves"]).cpu().numpy()
         vis = torch.stack(h["visits"]).cpu().numpy()

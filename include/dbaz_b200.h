@@ -187,6 +187,13 @@ int dbaz_selfplay_pick(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, uint64
  * games; move_idx is then not advanced) whose game goes on get reads = reads_by_k[legal moves] and their noise row times the
  * legal mask (mcts.py:223); the others get reads = -3.  Follow with dbaz_search_begin(reads, noise_buf, ...). */
 int dbaz_selfplay_restart(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, int32_t first, uint64_t stream);
+/* Optional, after dbaz_selfplay_restart and before dbaz_search_begin (same `first`): adjudication with the exact endgame
+ * solver below.  A tree that restarted (moves[t] >= 0, or first != 0) with searching[t] == 1 and whose root has at most
+ * max_free (0 .. 16) free real edges ends its game there: margin[t] = the root's final margin (int8, seen by its player
+ * to move), searching[t] = 0, reads[t] = -3 and *left is decremented, so that *left still counts the games going on.
+ * margin[t] of every other tree is not written (initialise it to -128).  Capturable in a CUDA graph. */
+int dbaz_selfplay_adjudicate(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, int8_t *margin, int32_t max_free,
+                             int32_t first, uint64_t stream);
 /* Synchronises `stream`.  out int64[8] = {trees with an error flag, total sims, total path nodes,
  * largest node-pool use of any tree (now or at a re-root), terminal leaves, eval-cache hits, 0, 0} (since reset_roots).  Returns non-zero (and sets
  * last_error) if any tree faulted. */
