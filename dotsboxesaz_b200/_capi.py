@@ -89,7 +89,9 @@ SYMBOLS = {
     "dbaz_solver_eval": (C.c_int, [_P, _P, _P, _P, _P, _I32, _I64, _U64]),
     "dbaz_endgame_moves": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _U64]),
     "dbaz_endgame_eval": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _I64, _U64]),
+    "dbaz_endgame_deep_moves": (C.c_int, [_P, _P, _I64, _I32, _P, _I64, _P, _P, _U64]),
 }
+ENDGAME_DEEP_GEOM_BYTES = 512  # workspace bytes of one position's geometry in dbaz_endgame_deep_moves, beside its 2^f table
 
 _lib = None
 

@@ -994,6 +994,82 @@ int dbaz_endgame_eval(dbaz_engine* e, const dbaz_state* leaf_states, float* prio
     return launch_ok(e, "k_endgame_eval");
 }
 
+int dbaz_endgame_deep_moves(dbaz_engine* e, const dbaz_state* states, int64_t n, int32_t f, int8_t* workspace, int64_t workspace_bytes,
+                            int8_t* move_margin, int8_t* margin, uint64_t stream) {
+    if (!e) return 1;
+    char buf[192];
+    if (f < ENDGAME_DEEP_MIN_FREE || f > ENDGAME_DEEP_MAX_FREE) {
+        std::snprintf(buf, sizeof buf, "dbaz_endgame_deep_moves: f must be in [%d, %d], got %d", ENDGAME_DEEP_MIN_FREE,
+                      ENDGAME_DEEP_MAX_FREE, f);
+        return fail(e, buf);
+    }
+    const int64_t per_position = ((int64_t)1 << f) + ENDGAME_DEEP_GEOM_BYTES;
+    if (workspace_bytes < per_position) {
+        std::snprintf(buf, sizeof buf, "dbaz_endgame_deep_moves: one position with f = %d needs 2^%d + %d = %lld workspace bytes, got %lld",
+                      f, f, ENDGAME_DEEP_GEOM_BYTES, (long long)per_position, (long long)workspace_bytes);
+        return fail(e, buf);
+    }
+    if (!states || !workspace || !move_margin || !margin) return fail(e, "dbaz_endgame_deep_moves: null buffer");
+    if (n < 0) {
+        std::snprintf(buf, sizeof buf, "dbaz_endgame_deep_moves: n must be >= 0, got %lld", (long long)n);
+        return fail(e, buf);
+    }
+    if (n == 0) return 0;
+    DeviceGuard guard(e->cfg.device);
+    const cudaStream_t st = S(stream);
+    const Board& b = e->board;
+    const int64_t pass = std::min<int64_t>(workspace_bytes / per_position, ENDGAME_DEEP_MAX_PASS);
+    unsigned long long* d_count = nullptr;
+    DBAZ_CK(e, cudaMalloc(&d_count, sizeof(unsigned long long)));
+    // per pass: tables to the sentinel, geometry (+ mismatch count), layers f-1 .. 0, one check over the pass's tables,
+    // then the outputs; a pass with a mismatched state is not solved, and the later passes only count
+    unsigned long long mismatch = 0, left = 0;
+    cudaError_t cst = cudaSuccess;
+    const char* what = "dbaz_endgame_deep_moves";
+    for (int64_t p0 = 0; p0 < n && cst == cudaSuccess && !left; p0 += pass) {
+        const int P = (int)std::min<int64_t>(pass, n - p0);
+        const int64_t bytes = (int64_t)P << f;
+        unsigned long long h = 0;
+        if ((cst = cudaMemsetAsync(workspace, 0x80, (size_t)bytes, st)) != cudaSuccess) break;
+        if ((cst = cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), st)) != cudaSuccess) break;
+        k_deep_geom<<<blocks_for((int64_t)P * 32, 256), 256, 0, st>>>(b, e->ta.act_tab, states + p0, workspace, f, P, d_count);
+        if ((cst = cudaGetLastError()) != cudaSuccess) { what = "k_deep_geom"; break; }
+        if ((cst = cudaMemcpyAsync(&h, d_count, sizeof h, cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
+        if ((cst = cudaStreamSynchronize(st)) != cudaSuccess) break;
+        mismatch += h;
+        if (mismatch) continue;
+        for (int k = f - 1; k >= 0 && cst == cudaSuccess; --k) {
+            const uint32_t count = c_binom_host(f, k);
+            k_deep_layer<<<dim3((unsigned)blocks_for(count, 256), (unsigned)P), 256, 0, st>>>(workspace, f, P, k, count);
+            if ((cst = cudaGetLastError()) != cudaSuccess) what = "k_deep_layer";
+        }
+        if (cst != cudaSuccess) break;
+        if ((cst = cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), st)) != cudaSuccess) break;
+        const int64_t n16 = bytes / 16;
+        k_solver_check<<<(int)std::min<int64_t>(blocks_for(n16, 256), (int64_t)e->n_sms * 8), 256, 0, st>>>(
+            reinterpret_cast<const uint4*>(workspace), n16, d_count);
+        if ((cst = cudaGetLastError()) != cudaSuccess) { what = "k_solver_check"; break; }
+        if ((cst = cudaMemcpyAsync(&left, d_count, sizeof left, cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
+        if ((cst = cudaStreamSynchronize(st)) != cudaSuccess) break;
+        if (left) break;
+        k_deep_moves<<<blocks_for((int64_t)P * 32, 256), 256, 0, st>>>(b, states + p0, workspace, f, P, move_margin + p0 * b.A,
+                                                                       margin + p0);
+        if ((cst = cudaGetLastError()) != cudaSuccess) { what = "k_deep_moves"; break; }
+    }
+    if (cst == cudaSuccess) cst = cudaStreamSynchronize(st);
+    cudaFree(d_count);
+    if (cst != cudaSuccess) return cuda_fail(e, what, cst);
+    if (mismatch) {
+        std::snprintf(buf, sizeof buf, "dbaz_endgame_deep_moves: %llu of %lld states do not have f = %d free edges", mismatch, (long long)n, f);
+        return fail(e, buf);
+    }
+    if (left) {
+        std::snprintf(buf, sizeof buf, "dbaz_endgame_deep_moves: %llu table entries were never written", left);
+        return fail(e, buf);
+    }
+    return 0;
+}
+
 int dbaz_selfplay_adjudicate(dbaz_engine* e, const dbaz_selfplay_buffers* bufs, int8_t* margin, int32_t max_free, int32_t first,
                              uint64_t stream) {
     if (!e || !bufs) return 1;

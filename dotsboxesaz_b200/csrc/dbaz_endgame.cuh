@@ -70,26 +70,20 @@ __device__ __forceinline__ uint32_t endgame_local(uint64_t F0, uint64_t F1, uint
     return m;
 }
 
-// Whole warp: the row's free edges and lead, and geo[i] = the local masks of the (up to) two boxes local edge i borders
-// (low / high 16 bits, from act_tab) for i < f <= 16.  d = LC - btc2[to_play] - closed boxes; box (l, c) is the second box
-// of its top edge l * cols + c.
-__device__ __forceinline__ EndgameRow endgame_row(const Board& b, const uint4* __restrict__ act_tab, const dbaz_state& s,
-                                                  uint32_t* geo, int lane) {
-    EndgameRow p;
-    p.F0 = b.real[0] & ~s.edges[0];
-    p.F1 = b.real[1] & ~s.edges[1];
-    const int f0 = __popcll(p.F0);
-    p.f = f0 + __popcll(p.F1);
-    if (lane < p.f && lane < ENDGAME_MAX_FREE) {
-        const int a = lane < f0 ? nth_set_bit(p.F0, lane) : 64 + nth_set_bit(p.F1, lane - f0);
-        uint32_t eb = 0;
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-            const uint4 q = __ldg(act_tab + 2 * a + k);
-            eb |= endgame_local(p.F0, p.F1, (uint64_t)q.x | ((uint64_t)q.y << 32), (uint64_t)q.z | ((uint64_t)q.w << 32)) << (16 * k);
-        }
-        geo[lane] = eb;
-    }
+// action of local edge i (f0 = free edges in word 0)
+__device__ __forceinline__ int endgame_action(uint64_t F0, uint64_t F1, int f0, int i) {
+    return i < f0 ? nth_set_bit(F0, i) : 64 + nth_set_bit(F1, i - f0);
+}
+
+// local mask of box k (0 or 1, from act_tab) of action a: its free edges (0 for no box)
+__device__ __forceinline__ uint32_t endgame_edge_box(const uint4* __restrict__ act_tab, uint64_t F0, uint64_t F1, int a, int k) {
+    const uint4 q = __ldg(act_tab + 2 * a + k);
+    return endgame_local(F0, F1, (uint64_t)q.x | ((uint64_t)q.y << 32), (uint64_t)q.z | ((uint64_t)q.w << 32));
+}
+
+// Whole warp: the mover's lead d = LC - btc2[to_play] - closed boxes; box (l, c) is the second box of its top edge
+// l * cols + c.
+__device__ __forceinline__ int endgame_lead(const Board& b, const uint4* __restrict__ act_tab, const dbaz_state& s, int lane) {
     int closed = 0;
     for (int x = lane; x < b.nboxes; x += 32) {
         const int l = x / b.C, c = x - l * b.C;
@@ -99,7 +93,26 @@ __device__ __forceinline__ EndgameRow endgame_row(const Board& b, const uint4* _
     }
     closed = __reduce_add_sync(0xffffffffu, closed);
     const int mine2 = (s.to_play & 1) ? s.btc2[1] : s.btc2[0];
-    p.d = b.nboxes - mine2 - closed;
+    return b.nboxes - mine2 - closed;
+}
+
+// Whole warp: the row's free edges and lead, and geo[i] = the local masks of the (up to) two boxes local edge i borders
+// (low / high 16 bits) for i < f <= 16.
+__device__ __forceinline__ EndgameRow endgame_row(const Board& b, const uint4* __restrict__ act_tab, const dbaz_state& s,
+                                                  uint32_t* geo, int lane) {
+    EndgameRow p;
+    p.F0 = b.real[0] & ~s.edges[0];
+    p.F1 = b.real[1] & ~s.edges[1];
+    const int f0 = __popcll(p.F0);
+    p.f = f0 + __popcll(p.F1);
+    if (lane < p.f && lane < ENDGAME_MAX_FREE) {
+        const int a = endgame_action(p.F0, p.F1, f0, lane);
+        uint32_t eb = 0;
+#pragma unroll
+        for (int k = 0; k < 2; ++k) eb |= endgame_edge_box(act_tab, p.F0, p.F1, a, k) << (16 * k);
+        geo[lane] = eb;
+    }
+    p.d = endgame_lead(b, act_tab, s, lane);
     return p;
 }
 
@@ -267,6 +280,94 @@ __global__ void __launch_bounds__(ENDGAME_THREADS, 3) k_endgame_eval(Board b, co
                                                                  const uint16_t* __restrict__ order, const dbaz_state* __restrict__ leaves,
                                                                  EndgameEvalOut out, int max_free, int64_t n) {
     endgame_rows(b, act_tab, order, StateRows{leaves}, out, max_free, n);
+}
+
+// ---- deep tier (DESIGN.md §13): positions with 17 <= f <= 32 free edges, one 2^f-byte table per position in device
+// memory, solved by the layer body of k_solver_layer over local edges.  A pass of P positions, all with the same f, uses
+// a caller-owned workspace: table p at ws + p 2^f, then geometry slot p at ws + P 2^f + p ENDGAME_DEEP_GEOM_BYTES.
+constexpr int ENDGAME_DEEP_MIN_FREE = ENDGAME_MAX_FREE + 1;
+constexpr int ENDGAME_DEEP_MAX_FREE = SOLVER_MAX_EDGES;
+constexpr int ENDGAME_DEEP_GEOM_BYTES = 512;
+constexpr int ENDGAME_DEEP_MAX_PASS = 65535;  // positions per pass: gridDim.y of k_deep_layer
+
+// One position's geometry in SolverGeom's shape: E = f and ebox = the local box masks of its free edges (act, box, LC and
+// nboxes are not used), plus the mover's lead.
+struct DeepGeom {
+    SolverGeom g;
+    int d;
+};
+static_assert(sizeof(DeepGeom) <= ENDGAME_DEEP_GEOM_BYTES, "a deep geometry slot holds a DeepGeom");
+
+__device__ __forceinline__ DeepGeom* deep_geom(int8_t* ws, int f, int P, int p) {
+    return reinterpret_cast<DeepGeom*>(ws + ((int64_t)P << f) + (int64_t)p * ENDGAME_DEEP_GEOM_BYTES);
+}
+
+// One warp per position of the pass: its geometry and the full-set entry T_p[2^f - 1] = 0 (the rest of the tables is the
+// sentinel).  A state whose f is not the launch's is counted in *mismatch and gets an empty geometry.
+__global__ void k_deep_geom(Board b, const uint4* __restrict__ act_tab, const dbaz_state* __restrict__ states, int8_t* ws, int f, int P,
+                            unsigned long long* __restrict__ mismatch) {
+    const int p = (int)((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (p >= P) return;
+    const dbaz_state s = states[p];
+    const uint64_t F0 = b.real[0] & ~s.edges[0], F1 = b.real[1] & ~s.edges[1];
+    const int f0 = __popcll(F0);
+    const bool ok = f0 + __popcll(F1) == f;
+    DeepGeom* G = deep_geom(ws, f, P, p);
+    uint32_t eb[2] = {0u, 0u};
+    if (ok && lane < f) {
+        const int a = endgame_action(F0, F1, f0, lane);
+        eb[0] = endgame_edge_box(act_tab, F0, F1, a, 0);
+        eb[1] = endgame_edge_box(act_tab, F0, F1, a, 1);
+    }
+    G->g.ebox[lane][0] = eb[0];
+    G->g.ebox[lane][1] = eb[1];
+    const int d = endgame_lead(b, act_tab, s, lane);
+    if (lane == 0) {
+        G->g.E = f;
+        G->d = d;
+        ws[((int64_t)p << f) + (((int64_t)1 << f) - 1)] = 0;
+        if (!ok) atomicAdd(mismatch, 1ull);
+    }
+}
+
+// Layer k of every table of the pass: blockIdx.y = position, blockIdx.x * 256 + threadIdx.x = entry of the layer.
+__global__ void __launch_bounds__(256) k_deep_layer(int8_t* ws, int f, int P, int k, uint32_t count) {
+    __shared__ SolverGeom g;
+    const int p = blockIdx.y;
+    const DeepGeom* G = deep_geom(ws, f, P, p);
+    if (threadIdx.x < 2 * SOLVER_MAX_EDGES) g.ebox[threadIdx.x >> 1][threadIdx.x & 1] = G->g.ebox[threadIdx.x >> 1][threadIdx.x & 1];
+    if (threadIdx.x == 0) g.E = f;
+    __syncthreads();
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    solver_layer_entry(g, ws + ((int64_t)p << f), k, r);
+}
+
+// One warp per position of the pass, from its filled table: move margins [P][A] and final margins [P] as k_endgame_moves.
+// A box closes iff local edge i is its last free edge (ebox == 1 << i).
+__global__ void k_deep_moves(Board b, const dbaz_state* __restrict__ states, int8_t* ws, int f, int P, int8_t* __restrict__ move_margin,
+                             int8_t* __restrict__ margin) {
+    const int p = (int)((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    if (p >= P) return;
+    const dbaz_state s = states[p];
+    const uint64_t F0 = b.real[0] & ~s.edges[0], F1 = b.real[1] & ~s.edges[1];
+    const DeepGeom* G = deep_geom(ws, f, P, p);
+    const int8_t* T = ws + ((int64_t)p << f);
+    const int d = G->d;
+    for (int a = lane; a < b.A; a += 32) {
+        int mm = SOLVER_SENTINEL;
+        if (a < 64 ? ((F0 >> a) & 1ull) : ((F1 >> (a - 64)) & 1ull)) {
+            const int i = endgame_rank(F0, F1, a);
+            const uint32_t bit = 1u << i;
+            const int c = (G->g.ebox[i][0] == bit ? 1 : 0) + (G->g.ebox[i][1] == bit ? 1 : 0);
+            const int v = T[bit];
+            mm = d + (c ? c + v : -v);
+        }
+        move_margin[(int64_t)p * b.A + a] = (int8_t)mm;
+    }
+    if (lane == 0) margin[p] = (int8_t)(d + T[0]);
 }
 
 }  // namespace dbaz

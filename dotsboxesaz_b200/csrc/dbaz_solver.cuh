@@ -70,12 +70,10 @@ __device__ __forceinline__ uint32_t solver_full(const SolverGeom& g) {
     return g.E == 32 ? 0xffffffffu : ((1u << g.E) - 1u);
 }
 
-// Layer k of the table: thread r solves the r-th k-subset in colex order, so consecutive threads write increasing masks
-// and their reads M | 1 << j of small j fall into shared sectors.  Layer k + 1 is complete (previous launch).
-__global__ void __launch_bounds__(256) k_solver_layer(const __grid_constant__ SolverGeom g, int8_t* __restrict__ T, int k,
-                                                      uint32_t count) {
-    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= count) return;
+// Entry r of layer k of a table over g.E edges: the r-th k-subset in colex order, so consecutive threads write increasing
+// masks and their reads M | 1 << j of small j fall into shared sectors.  Layer k + 1 is complete (previous launch).
+// One body for the full-board table (k_solver_layer) and the per-position tables of dbaz_endgame.cuh (k_deep_layer).
+__device__ __forceinline__ void solver_layer_entry(const SolverGeom& g, int8_t* __restrict__ T, int k, uint32_t r) {
     const uint32_t M = colex_unrank(r, k, g.E);
     uint32_t fr = solver_full(g) & ~M;
     int best = SOLVER_SENTINEL;
@@ -88,6 +86,14 @@ __global__ void __launch_bounds__(256) k_solver_layer(const __grid_constant__ So
         best = max(best, c ? c + v : -v);
     }
     T[M] = (int8_t)best;
+}
+
+// Layer k of the full-board table.
+__global__ void __launch_bounds__(256) k_solver_layer(const __grid_constant__ SolverGeom g, int8_t* __restrict__ T, int k,
+                                                      uint32_t count) {
+    const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    solver_layer_entry(g, T, k, r);
 }
 
 // Number of sentinel bytes left in the table (16 bytes per thread and step; 2^E is a multiple of 16 for E >= 4).

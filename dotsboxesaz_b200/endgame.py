@@ -5,16 +5,19 @@ A position with f free edges is solved by a retrograde over the 2^f subsets of t
 margin, outcome and move margins are those of the 32-edge table of solver.py, which the two must agree on byte for byte.
 No table is kept, and nothing needs solving up front.
 
-EndgameSolver     per-state queries: margins, outcomes, move margins, optimal moves, which states are solvable.
-EndgameEvaluator  wraps any evaluator: exact priors and values on the leaves that are solvable, the inner evaluator's
-                  output on every other leaf.
-solver.grade / solver.grade_samples take an EndgameSolver too and grade the solvable rows.
+EndgameSolver       per-state queries: margins, outcomes, move margins, optimal moves, which states are solvable.
+DeepEndgameSolver   the same queries up to f <= 32 (DESIGN.md §13): positions with 17 <= f free edges are solved in a
+                    2^f-byte table each in device memory, outside CUDA graphs.
+EndgameEvaluator    wraps any evaluator: exact priors and values on the leaves that are solvable, the inner evaluator's
+                    output on every other leaf.
+solver.grade / solver.grade_samples take either endgame solver too and grade the solvable rows.
 """
 import ctypes as C
 
+import numpy as np
 import torch
 
-from ._capi import RESULT_NONE
+from ._capi import ENDGAME_DEEP_GEOM_BYTES, RESULT_NONE
 from .engine import EngineError, _ptr
 from .solver import ILLEGAL
 
@@ -144,6 +147,59 @@ class EndgameSolver:
         return words
 
 
+SHALLOW_MAX_FREE = 16  # the shared-memory tier of EndgameSolver
+
+
+class DeepEndgameSolver(EndgameSolver):
+    """EndgameSolver up to `max_free` (17 .. 32) free edges.  Rows with f <= 16 are solved as by EndgameSolver(engine, 16),
+    rows with 17 <= f <= max_free by dbaz_endgame_deep_moves (grouped by f, one 2^f-byte table per position in a
+    workspace of `workspace_bytes`, allocated at the first deep query and kept; default: max(one position at max_free,
+    1 GiB)), every other row reads ILLEGAL.  A position costs about f 2^(f-1) successor reads.
+    Every query synchronises the host (it reads the rows' f and the solver's checks), so it cannot be captured in a CUDA
+    graph: evaluate / adjudicate raise ValueError, and EndgameEvaluator does not take it."""
+
+    def __init__(self, engine, max_free=24, workspace_bytes=None):
+        max_free = int(max_free)
+        if not SHALLOW_MAX_FREE < max_free <= 32:
+            raise ValueError("max_free must be in [17, 32], got %d" % max_free)
+        need = (1 << max_free) + ENDGAME_DEEP_GEOM_BYTES
+        workspace_bytes = max(need, 1 << 30) if workspace_bytes is None else int(workspace_bytes)
+        if workspace_bytes < need:
+            raise ValueError("one position with %d free edges needs %d workspace bytes, got %d" % (max_free, need, workspace_bytes))
+        super().__init__(engine, max_free)
+        self.workspace_bytes = workspace_bytes
+        self.workspace = None
+
+    def moves(self, states):
+        """(move margins int8 [n, A] with ILLEGAL for played edges and padding, final margins int8 [n]); every byte of a
+        row with f > max_free is ILLEGAL.  Synchronises."""
+        eng = self.eng
+        states = eng._states_arg(states)
+        n = states.shape[0]
+        mm = torch.empty((n, self.A), dtype=torch.int8, device=eng.device)
+        mg = torch.empty((n,), dtype=torch.int8, device=eng.device)
+        self._ck(eng.lib.dbaz_endgame_moves(eng._h, _ptr(states), _ptr(mm), _ptr(mg), SHALLOW_MAX_FREE, n, eng._stream()))
+        f = self.free_edges(states).cpu().numpy()
+        for fv in np.unique(f[(f > SHALLOW_MAX_FREE) & (f <= self.max_free)]):
+            idx = torch.from_numpy(np.flatnonzero(f == fv)).to(eng.device)
+            sub = states[idx].contiguous()
+            smm = torch.empty((sub.shape[0], self.A), dtype=torch.int8, device=eng.device)
+            smg = torch.empty((sub.shape[0],), dtype=torch.int8, device=eng.device)
+            if self.workspace is None:
+                self.workspace = torch.empty((self.workspace_bytes,), dtype=torch.int8, device=eng.device)
+            self._ck(eng.lib.dbaz_endgame_deep_moves(eng._h, _ptr(sub), sub.shape[0], int(fv), _ptr(self.workspace), self.workspace_bytes,
+                                                     _ptr(smm), _ptr(smg), eng._stream()))
+            mm[idx] = smm
+            mg[idx] = smg
+        return mm, mg
+
+    def evaluate(self, *args, **kwargs):
+        raise ValueError("DeepEndgameSolver synchronises the host and cannot run inside the search; use EndgameSolver (max_free <= 16)")
+
+    def adjudicate(self, *args, **kwargs):
+        raise ValueError("DeepEndgameSolver synchronises the host and cannot run inside self-play; use EndgameSolver (max_free <= 16)")
+
+
 class EndgameEvaluator:
     """`inner` (FakeNetEvaluator, an nn plan, SolverEvaluator, ...) followed by one k_endgame_eval over the same leaves:
     exact values on the leaves with at most endgame.max_free free edges, and exact priors there unless priors="inner".
@@ -156,6 +212,8 @@ class EndgameEvaluator:
             raise ValueError("value must be 'outcome' or 'margin'")
         if priors not in ("exact", "inner"):
             raise ValueError("priors must be 'exact' or 'inner'")
+        if isinstance(endgame, DeepEndgameSolver):
+            raise ValueError("the evaluator runs inside the search's CUDA graphs; DeepEndgameSolver cannot, use EndgameSolver")
         self.inner = inner
         self.endgame = endgame
         self.mode = 0 if value == "outcome" else 1

@@ -190,12 +190,15 @@ def grade_samples(solver, batch):
     return grade(solver, solver.states_from_planes(batch.planes), policy=batch.pi, z=batch.z)
 
 
-def play_vs_solver(engine, evaluator, params, solver, n_games, seed=0):
+def play_vs_solver(engine, evaluator, params, solver, n_games, seed=0, start_states=None):
     """`n_games` lock-step games of a model against the perfect opponent, in the style of self_play.compute_elo: the
     model plays player 0 in even games and player 1 in odd ones; its moves come from Engine.run_search with
     params.self_play (budget, PUCT constants, Dirichlet noise, temperature schedule, tree reuse), on trees where the
     solver is to move the search is idle; the solver plays a uniformly random margin-optimal move.  Both sides' draws
     come from one device generator seeded with `seed`.
+    start_states (int64 [n_games, 4], optional): the games start there instead of the empty board; move numbers (the
+    temperature schedule) count from there.  With an endgame solver every start state must be solvable.  Each model
+    search gets _n_searches(legal moves of its root) simulations.
     Returns dict(wins, draws, losses, model_moves, blunders) -- a blunder is a model move whose margin has a lower sign
     than the outcome of the position it was played from -- plus, on the device: result int8 [n_games] (the model's
     result), states [plies, n_games, 4], moves int32 [plies, n_games] (-1 once a game is over) and model bool
@@ -210,8 +213,17 @@ def play_vs_solver(engine, evaluator, params, solver, n_games, seed=0):
     dev = eng.device
     num_read = sp.mcts.mcts_num_read
     alpha, coeff = sp.noise
+    roots0 = None
+    if start_states is not None:
+        start_states = eng._states_arg(start_states)
+        if start_states.shape[0] != n_games:
+            raise ValueError("start_states must have n_games rows")
+        if hasattr(solver, "max_free") and not bool(solver.solvable(start_states).all()):
+            raise ValueError("every start state must have at most max_free = %d free edges" % solver.max_free)
+        roots0 = eng.new_states(n)
+        roots0[:n_games] = start_states
     eng.set_cpuct(sp.mcts.mcts_cpuct)
-    eng.reset_roots()
+    eng.reset_roots(roots0)
     slot = torch.arange(n, device=dev)
     playing = slot < n_games
     model_player = slot % 2
@@ -231,9 +243,10 @@ def play_vs_solver(engine, evaluator, params, solver, n_games, seed=0):
         to_play = roots.view(torch.uint8).reshape(n, 32)[:, 20].long()
         model_turn = active & (to_play == model_player)
         valid = eng.valid_moves(roots)
-        budget = _n_searches(solver.E - move_i, num_read)  # one edge per move: E - move_i legal moves left
-        reads = torch.where(model_turn, torch.full((n,), budget, dtype=torch.int32, device=dev),
-                            torch.full((n,), -1, dtype=torch.int32, device=dev))
+        legal = valid.sum(1).cpu().tolist()
+        budgets = torch.tensor([_n_searches(int(k), num_read) for k in legal], dtype=torch.int32, device=dev)
+        budget = int(budgets[active].max())
+        reads = torch.where(model_turn, budgets, torch.full((n,), -1, dtype=torch.int32, device=dev))
         noise = None
         if alpha > 0:
             g_ = torch._standard_gamma(torch.full((n, eng.A), float(alpha), dtype=torch.float64, device=dev), generator=gen)

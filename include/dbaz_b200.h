@@ -356,6 +356,15 @@ int dbaz_endgame_moves(dbaz_engine *e, const dbaz_state *states, int8_t *move_ma
  * margin / (L C) (mode 1).  Every other row keeps its bits.  A function of the eval-cache key. */
 int dbaz_endgame_eval(dbaz_engine *e, const dbaz_state *leaf_states, float *priors, float *values, int32_t mode,
                       int32_t keep_priors, int32_t max_free, int64_t n, uint64_t stream);
+/* Deep tier (DESIGN.md §13): every one of the n states has exactly f free real edges, 17 <= f <= 32.  Each is solved in a
+ * 2^f-byte table of its own in the caller-owned device workspace, by the layer kernel of dbaz_solver_solve over its free
+ * edges; a position takes 2^f + 512 bytes of workspace (table and geometry), and the states are solved in passes of as
+ * many positions as the workspace holds (at most 65 535).  Outputs as dbaz_endgame_moves: move_margin int8[n][A] (-128
+ * for played edges and padding) and margin int8[n].  Rejects f outside [17, 32], a workspace smaller than one position,
+ * null buffers, n < 0, states whose f differs and unwritten table entries.  Allocates an 8-byte counter and synchronises
+ * `stream`; not capturable. */
+int dbaz_endgame_deep_moves(dbaz_engine *e, const dbaz_state *states, int64_t n, int32_t f, int8_t *workspace,
+                            int64_t workspace_bytes, int8_t *move_margin, int8_t *margin, uint64_t stream);
 
 #ifdef __cplusplus
 }
