@@ -66,6 +66,7 @@ SYMBOLS = {
     "dbaz_selfplay_pick": (C.c_int, [_P, C.POINTER(SelfplayBuffers), _U64]),
     "dbaz_selfplay_restart": (C.c_int, [_P, C.POINTER(SelfplayBuffers), _I32, _U64]),
     "dbaz_selfplay_adjudicate": (C.c_int, [_P, C.POINTER(SelfplayBuffers), _P, _I32, _I32, _U64]),
+    "dbaz_selfplay_exact_endgame": (C.c_int, [_P, C.POINTER(SelfplayBuffers), _P, _I32, _I32, _I32, _U64]),
     "dbaz_search_status": (C.c_int, [_P, _P, _U64]),
     "dbaz_search_set_mode": (C.c_int, [_P, _I32, _I32]),
     "dbaz_search_set_chain_budget": (C.c_int, [_P, _I32]),

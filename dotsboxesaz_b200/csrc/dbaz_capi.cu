@@ -40,7 +40,8 @@ struct dbaz_engine {
     int solver_edges;     // real edges of the board (E)
     SolverGeom sg;        // compact geometry of the exact solver, valid when solver_edges <= SOLVER_MAX_EDGES
     uint16_t* eg_order;   // endgame_order_host: the masks of every f <= 16 by popcount (ENDGAME_ORDER_ENTRIES)
-    int eg_blocks[3][ENDGAME_MAX_FREE + 1];  // resident CTAs per SM of k_endgame_moves / k_endgame_eval / k_selfplay_adjudicate by max_free
+    int eg_blocks[4][ENDGAME_MAX_FREE + 1];  // resident CTAs per SM of k_endgame_moves / k_endgame_eval / k_selfplay_adjudicate /
+                                             // k_selfplay_exact_endgame by max_free
     std::string err;
 };
 
@@ -190,8 +191,9 @@ static cudaError_t build_endgame(dbaz_engine* e) {
     endgame_order_host(order.data());
     cudaError_t st = cudaMalloc(&e->eg_order, order.size() * sizeof(uint16_t));
     if (st == cudaSuccess) st = cudaMemcpy(e->eg_order, order.data(), order.size() * sizeof(uint16_t), cudaMemcpyHostToDevice);
-    const void* kernels[3] = {(const void*)k_endgame_moves, (const void*)k_endgame_eval, (const void*)k_selfplay_adjudicate};
-    for (int k = 0; k < 3 && st == cudaSuccess; ++k) {
+    const void* kernels[4] = {(const void*)k_endgame_moves, (const void*)k_endgame_eval, (const void*)k_selfplay_adjudicate,
+                              (const void*)k_selfplay_exact_endgame};
+    for (int k = 0; k < 4 && st == cudaSuccess; ++k) {
         st = cudaFuncSetAttribute(kernels[k], cudaFuncAttributeMaxDynamicSharedMemorySize, endgame_smem_bytes(ENDGAME_MAX_FREE));
         for (int f = 0; f <= ENDGAME_MAX_FREE && st == cudaSuccess; ++f) {
             int nb = 0;
@@ -1081,6 +1083,20 @@ int dbaz_selfplay_adjudicate(dbaz_engine* e, const dbaz_selfplay_buffers* bufs, 
     k_selfplay_adjudicate<<<endgame_grid(e, 2, max_free, e->ta.n_trees), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
         e->board, e->ta, e->eg_order, sp, margin, max_free, first ? 1 : 0);
     return launch_ok(e, "k_selfplay_adjudicate");
+}
+
+int dbaz_selfplay_exact_endgame(dbaz_engine* e, const dbaz_selfplay_buffers* bufs, int8_t* exact_margin, int32_t max_free, int32_t kind,
+                                int32_t first, uint64_t stream) {
+    if (!e || !bufs) return 1;
+    if (endgame_bad_max_free(e, "dbaz_selfplay_exact_endgame", max_free)) return 1;
+    if (kind < 0 || kind > 1) return fail(e, "dbaz_selfplay_exact_endgame: kind must be 0 (outcome) or 1 (margin)");
+    if (!exact_margin) return fail(e, "dbaz_selfplay_exact_endgame: null exact_margin");
+    SelfplayArgs sp;
+    if (int rc = selfplay_args(e, bufs, sp)) return rc;
+    DeviceGuard guard(e->cfg.device);
+    k_selfplay_exact_endgame<<<endgame_grid(e, 3, max_free, e->ta.n_trees), ENDGAME_THREADS, endgame_smem_bytes(max_free), S(stream)>>>(
+        e->board, e->ta, e->eg_order, sp, exact_margin, max_free, kind, first ? 1 : 0);
+    return launch_ok(e, "k_selfplay_exact_endgame");
 }
 
 }  // extern "C"

@@ -13,6 +13,9 @@
 //   k_selfplay_adjudicate  optional, after the restart: a game whose new root has f <= max_free free edges ends there
 //                       with the exact final margin of that root (the endgame solver of dbaz_endgame.cuh); its root is
 //                       not searched and gives no sample.
+//   k_selfplay_exact_endgame  optional instead, at the same place: a game whose new root has f <= max_free free edges is
+//                       played out from there with optimal moves by the warp that solves the root, one sample row per
+//                       ply with the optimal moves as its visits, and ends with that root's exact final margin.
 #pragma once
 #include "dbaz_tree_kernels.cuh"
 #include "dbaz_endgame.cuh"
@@ -190,6 +193,94 @@ __global__ void __launch_bounds__(ENDGAME_THREADS, 3) k_selfplay_adjudicate(Boar
                                                                         SelfplayArgs sp, int8_t* margin, int max_free, int first) {
     endgame_rows(b, ta.act_tab, order, RootRows{ta, sp.searching, sp.moves, first},
                  AdjudicateOut{margin, sp.searching, sp.reads, sp.left}, max_free, (int64_t)ta.n_trees);
+}
+
+// A solvable qualifying root is played out to the end of its game by the warp that solved it, from that one table (DESIGN.md
+// §14).  Lane i is local edge i (f <= 16); m = the local edges played since the root, d = the mover's lead (as endgame_lead
+// reads it from the state: the boxes closed since the root are counted, the rest comes from btc2).  Per ply, the
+// row mi = move_idx[t] + j gets what k_selfplay_pick writes for a searched root: the published state, visits = 1 on the
+// optimal moves (kind 0: outcome-optimal, 1: margin-optimal) and 0 elsewhere, zero tree statistics and q, the move drawn
+// from uniforms[mi][t] with pick's arithmetic (weights 1.0: a running double sum, the first action beyond u * k, else the
+// last positive weight), active = 1.  The game ends at the first state with a result (or a full history).  Then the tree
+// ends as in AdjudicateOut, with move_idx[t] = its last row and exact_margin[t] = the root's final margin.  The tree's
+// node pool is not touched: its root stays the exact root.
+struct ExactOut {
+    TreeArgs ta;
+    SelfplayArgs sp;
+    int8_t* exact_margin;
+    int kind;
+    static constexpr bool kUnsolvable = false;
+    __device__ __forceinline__ void unsolvable(const Board&, int64_t, int) const {}
+    __device__ __forceinline__ void solved(const Board& b, const EndgameRow& p, const int8_t* T, const uint32_t* geo, int64_t tw,
+                                           int lane) const {
+        const int t = (int)tw, n = ta.n_trees, A = b.A;
+        const bool mine = lane < p.f;
+        const uint32_t bit = 1u << lane;
+        const int act = mine ? endgame_action(p.F0, p.F1, __popcll(p.F0), lane) : -1;
+        const uint32_t eb = mine ? geo[lane] : 0u, b0 = eb & 0xffffu, b1 = eb >> 16;
+        dbaz_state s = load_hdr(node_ptr(ta, t, 0));
+        const int64_t mi0 = sp.move_idx[t];
+        uint32_t m = 0;
+        int closed = b.nboxes - ((s.to_play & 1) ? s.btc2[1] : s.btc2[0]) - p.d;  // boxes closed at the root
+        int d = p.d, j = 0;
+        for (; state_result(s) == DBAZ_RESULT_NONE && mi0 + j < sp.n_moves; ++j) {
+            const int64_t row = (mi0 + j) * n + t;
+            const int vm = T[m];
+            int c = 0;
+            bool opt = false;
+            if (mine && !(m & bit)) {
+                const uint32_t x = m | bit;
+                c = ((b0 && (x & b0) == b0) ? 1 : 0) + ((b1 && (x & b1) == b1) ? 1 : 0);
+                const int v = T[x];
+                const int mv = c ? c + v : -v;
+                opt = kind ? mv == vm : sign_of(d + mv) == sign_of(d + vm);
+            }
+            const uint32_t om = __ballot_sync(0xffffffffu, opt);
+            if (!om) break;  // no free edge left without a result: only a state with inconsistent scores gets here
+            for (int a = lane; a < A; a += 32) {
+                const bool fr = a < 64 ? ((p.F0 >> a) & 1ull) : ((p.F1 >> (a - 64)) & 1ull);
+                sp.h_visits[row * A + a] = fr ? (int32_t)((om >> endgame_rank(p.F0, p.F1, a)) & 1u) : 0;
+            }
+            // local edges are in action order, so the running count of optimal local edges is pick's cdf
+            const double target = sp.uniforms[row] * (double)__popc(om);
+            const unsigned beyond = __ballot_sync(0xffffffffu, mine && (double)__popc(om & (bit | (bit - 1u))) > target);
+            const unsigned last = __ballot_sync(0xffffffffu, opt && (om >> lane) == 1u);  // the last optimal local edge
+            const int i = __ffs(beyond ? beyond : last) - 1;
+            const int move = __shfl_sync(0xffffffffu, act, i);
+            const int c_i = __shfl_sync(0xffffffffu, c, i);
+            if (lane == 0) {
+                dbaz_state pub = s;
+                pub.flags = 0; pub.depth = 0; pub.parent = -1; pub.parent_action = -1; pub.result = (int16_t)state_result(s);
+                sp.h_states[row] = pub;
+                int32_t* o = sp.h_stats + row * 8;
+#pragma unroll
+                for (int k = 0; k < 8; ++k) o[k] = 0;
+                sp.h_q[row] = 0.0f;
+                sp.h_moves[row] = move;
+                sp.h_active[row] = 1;
+            }
+            state_apply<2>(s, move, c_i);  // two edge words fit every board: the second stays 0 where A <= 64
+            closed += c_i;
+            d = b.nboxes - ((s.to_play & 1) ? s.btc2[1] : s.btc2[0]) - closed;
+            m |= 1u << i;
+        }
+        if (lane == 0) {
+            exact_margin[t] = (int8_t)(p.d + T[0]);
+            if (j > 0) sp.move_idx[t] = mi0 + j - 1;  // (no row: a root with a result or a full history, not met in self-play)
+            sp.searching[t] = 0;
+            sp.reads[t] = -3;
+            atomicSub(sp.left, 1);
+        }
+    }
+};
+
+// Two CTAs of 512 threads per SM, not the three of the other endgame kernels: the playout loop does not fit their 40
+// registers (it spilled there); it takes 59 here, without spills.
+__global__ void __launch_bounds__(ENDGAME_THREADS, 2) k_selfplay_exact_endgame(Board b, TreeArgs ta, const uint16_t* __restrict__ order,
+                                                                           SelfplayArgs sp, int8_t* exact_margin, int max_free,
+                                                                           int kind, int first) {
+    endgame_rows(b, ta.act_tab, order, RootRows{ta, sp.searching, sp.moves, first}, ExactOut{ta, sp, exact_margin, kind}, max_free,
+                 (int64_t)ta.n_trees);
 }
 
 }  // namespace dbaz

@@ -107,6 +107,17 @@ class EndgameSolver:
         eng = self.eng
         eng._ck(eng.lib.dbaz_selfplay_adjudicate(eng._h, C.byref(bufs), _ptr(margin), self.max_free, 1 if first else 0, eng._stream()))
 
+    def play_out(self, bufs, exact_margin, kind="outcome", first=False):
+        """dbaz_selfplay_exact_endgame, after Engine.selfplay_restart(bufs, first): every game of the asynchronous self-play
+        loop whose new root has at most max_free free edges is played out from there with optimal moves (kind "outcome" or
+        "margin"), one history row per ply with the optimal moves as its visits, and ends with the root's final margin in
+        exact_margin (int8 [n_games], ILLEGAL elsewhere)."""
+        eng = self.eng
+        if kind not in ("outcome", "margin"):
+            raise ValueError("kind must be 'outcome' or 'margin'")
+        eng._ck(eng.lib.dbaz_selfplay_exact_endgame(eng._h, C.byref(bufs), _ptr(exact_margin), self.max_free,
+                                                    0 if kind == "outcome" else 1, 1 if first else 0, eng._stream()))
+
     def full_states(self, n):
         """n states with every real edge played (f = 0)."""
         st = self.eng.new_states(n)
@@ -156,7 +167,7 @@ class DeepEndgameSolver(EndgameSolver):
     workspace of `workspace_bytes`, allocated at the first deep query and kept; default: max(one position at max_free,
     1 GiB)), every other row reads ILLEGAL.  A position costs about f 2^(f-1) successor reads.
     Every query synchronises the host (it reads the rows' f and the solver's checks), so it cannot be captured in a CUDA
-    graph: evaluate / adjudicate raise ValueError, and EndgameEvaluator does not take it."""
+    graph: evaluate / adjudicate / play_out raise ValueError, and EndgameEvaluator does not take it."""
 
     def __init__(self, engine, max_free=24, workspace_bytes=None):
         max_free = int(max_free)
@@ -198,6 +209,8 @@ class DeepEndgameSolver(EndgameSolver):
 
     def adjudicate(self, *args, **kwargs):
         raise ValueError("DeepEndgameSolver synchronises the host and cannot run inside self-play; use EndgameSolver (max_free <= 16)")
+
+    play_out = adjudicate
 
 
 class EndgameEvaluator:

@@ -41,13 +41,23 @@ def _n_searches(n_valid, num_read):
 def _game_outcomes(final, result, margin):
     """Per game (int8 tensors [n]): the player whose sample rows get z = +outcome, and the outcome; every other row of
     the game gets -outcome.  A game played out: just_played of its terminal state and its result.  A game adjudicated
-    at a root (margin != ILLEGAL, the root's final margin): that root's player to move and sign(margin)."""
+    at a root, or played out exactly from it by the asynchronous loop, whose tree keeps that root (margin != ILLEGAL,
+    the root's final margin): that root's player to move and sign(margin)."""
     from .solver import ILLEGAL
     raw = final.view(torch.uint8).reshape(-1, 32)
     adj = margin != ILLEGAL
     player = torch.where(adj, raw[:, 20], raw[:, 21]).to(torch.int8)
     outcome = torch.where(adj, torch.sign(margin), result.to(torch.int8))
     return player, outcome
+
+
+def _hist_outcomes(h):
+    """_game_outcomes of a device-resident history: adjudicated games (h["margin"]) and games played out exactly by the
+    asynchronous loop (h["exact_margin"]; the two modes exclude each other)."""
+    margin = h["margin"]
+    if h.get("exact_margin") is not None:
+        margin = torch.where(h["exact_margin"] != -128, h["exact_margin"], margin)
+    return _game_outcomes(h["final"], h["result"], margin)
 
 
 def _dataset(rows, generation, with_features):
@@ -157,9 +167,19 @@ class BatchedSelfPlay:
     evaluator to pair it with is EndgameEvaluator(inner, EndgameSolver(engine, m)) with m >= max_free, so that the net
     is never asked about the positions it no longer trains on (not enforced).  Games that end at a majority earlier are
     played as without adjudication.
+
+    exact_endgame (default: params.self_play.exact_endgame; None = off): max_free in 0 .. 16, the alternative to
+    adjudicate that keeps those positions (DESIGN.md §14).  From the first root that is still going on and has at most
+    max_free free edges, the game is played out without a search: every root gives a sample row whose visits are 1 on the
+    optimal moves and 0 elsewhere (so pi is uniform over them; exact_policy "outcome" or "margin" picks outcome- or
+    margin-optimal moves), with zero tree statistics and q, and the move is drawn from that row by the path's usual
+    draw law (temperature has no effect, no Dirichlet noise is drawn).  Every row's z is the played-out result, which
+    optimal play keeps equal to the root's exact outcome.  Up to that root a game is the same game as without the
+    mode.  adjudicate and exact_endgame exclude each other.
     """
 
-    def __init__(self, engine, evaluator, params, graph_waves=16, pending=None, adaptive=None, adjudicate=None):
+    def __init__(self, engine, evaluator, params, graph_waves=16, pending=None, adaptive=None, adjudicate=None, exact_endgame=None,
+                 exact_policy="outcome"):
         self.eng = engine
         self.ev = evaluator
         self.params = params
@@ -180,6 +200,18 @@ class BatchedSelfPlay:
             if not 0 <= int(m) <= 16:
                 raise ValueError("adjudicate must be a max_free in 0 .. 16 or None, got %r" % (m,))
             self.endgame = EndgameSolver(engine, int(m))
+        x = params.self_play.get("exact_endgame", None) if exact_endgame is None else exact_endgame
+        self.exact = None
+        self.exact_policy = exact_policy
+        if x is not None:
+            from .endgame import EndgameSolver
+            if not 0 <= int(x) <= 16:
+                raise ValueError("exact_endgame must be a max_free in 0 .. 16 or None, got %r" % (x,))
+            if self.endgame is not None:
+                raise ValueError("adjudicate and exact_endgame exclude each other: set one of them")
+            if exact_policy not in ("outcome", "margin"):
+                raise ValueError("exact_policy must be 'outcome' or 'margin', got %r" % (exact_policy,))
+            self.exact = EndgameSolver(engine, int(x))
 
     def play_games(self, games_idxs, seeds=None, start_states=None, with_features=True):
         eng, sp = self.eng, self.params.self_play
@@ -200,6 +232,8 @@ class BatchedSelfPlay:
         hist = [[] for _ in range(n)]  # per game: row dicts of every searched root
         moves_played = [[] for _ in range(n)]
         margin = np.full(n, -128, dtype=np.int8)  # final margin of the root a game was adjudicated at, -128 (ILLEGAL) if none
+        exact_seen = np.zeros(n, dtype=bool)      # games that reached exact play
+        exact_rows = 0
         move_i = -1
         while active.any():
             move_i += 1
@@ -217,22 +251,39 @@ class BatchedSelfPlay:
                     active &= ~due
             if not active.any():
                 break
+            due = np.zeros(n, dtype=bool)  # games in exact play: no search, visits = their optimal moves
+            if self.exact is not None:
+                due = active & (self.exact.free_edges(roots).cpu().numpy() <= self.exact.max_free)
+                if due.any():
+                    idx = np.flatnonzero(due)
+                    opt = np.zeros((n, A), dtype=np.int32)
+                    opt[idx] = self.exact.optimal_moves(roots[torch.from_numpy(idx).to(roots.device)].contiguous(),
+                                                        self.exact_policy).cpu().numpy()
+                    exact_seen |= due
+                    exact_rows += int(due.sum())
             reads = np.full(n, -1, dtype=np.int32)
             noise = np.zeros((n, A), dtype=np.float64) if alpha > 0 else None
             for g in np.flatnonzero(active):
                 if move_i in temp_sched:
                     temperature[g] = temp_sched[move_i]
+                if due[g]:
+                    continue
                 reads[g] = _n_searches(int(valid[g].sum()), num_read)
                 if alpha > 0:
                     noise[g] = rngs[g].dirichlet(np.ones(A) * alpha, 1).ravel() * valid[g]
-            eng.run_search(torch.from_numpy(reads), self.ev, noise=None if noise is None else torch.from_numpy(noise),
-                           coeff=coeff, max_reads=int(reads.max()), graph_waves=self.graph_waves, pending=self.pending,
-                           adaptive=self.adaptive)
+            if (reads >= 0).any():
+                eng.run_search(torch.from_numpy(reads), self.ev, noise=None if noise is None else torch.from_numpy(noise),
+                               coeff=coeff, max_reads=int(reads.max()), graph_waves=self.graph_waves, pending=self.pending,
+                               adaptive=self.adaptive)
             vis = eng.root_visits().cpu().numpy()
             stats, _rW, q = (x.cpu().numpy() for x in eng.tree_stats())
+            if due.any():
+                vis[due] = opt[due]
+                stats[due] = 0
+                q[due] = 0.0
             moves = np.full(n, -1, dtype=np.int32)
             for g in np.flatnonzero(active):
-                probs = _apply_temperature(vis[g], temperature[g])
+                probs = vis[g] / vis[g].sum() if due[g] else _apply_temperature(vis[g], temperature[g])
                 r = rngs[g]
                 moves[g] = r.choice(A, 1, p=probs)[0]
                 hist[g].append({"game_idx": games_idxs[g], "move_idx": move_i, "move": moves_played[g][-1] if moves_played[g] else None,
@@ -245,6 +296,8 @@ class BatchedSelfPlay:
         info = eng.status()
         self.total_sims = info["sims"]
         info["adjudicated"] = int((margin[:len(games_idxs)] != -128).sum())
+        info["exact_games"] = int(exact_seen[:len(games_idxs)].sum())
+        info["exact_rows"] = exact_rows
         final = eng.root_states()
         winners, outcomes = (x.cpu().numpy() for x in _game_outcomes(final, eng.result(final), torch.from_numpy(margin).to(final.device)))
         for g in range(len(games_idxs)):
@@ -287,7 +340,10 @@ class BatchedSelfPlay:
         temperature = None
         hist_states, hist_visits, hist_active, hist_moves, hist_stats, hist_q = [], [], [], [], [], []
         margin = torch.full((n,), -128, dtype=torch.int8, device=dev)  # final margin of an adjudicated game's root, else ILLEGAL
-        full = self.endgame.full_states(n) if self.endgame is not None else None
+        solver = self.endgame if self.endgame is not None else self.exact
+        full = solver.full_states(n) if solver is not None else None
+        exact_seen = torch.zeros((n,), dtype=torch.bool, device=dev)     # games that reached exact play
+        exact_rows = torch.zeros((), dtype=torch.int64, device=dev)
         for move_i in range(n_moves):
             if move_i in temp_sched:
                 temperature = float(temp_sched[move_i])
@@ -300,14 +356,26 @@ class BatchedSelfPlay:
                 due = active & (self.endgame.free_edges(roots) <= self.endgame.max_free)
                 margin = torch.where(due, self.endgame.margin(torch.where(due.unsqueeze(1), roots, full).contiguous()), margin)
                 active &= ~due
+            exact = None
+            if self.exact is not None:
+                # roots in exact play: not searched, their visit row is their optimal moves (the other rows solve the full board)
+                exact = active & (self.exact.free_edges(roots) <= self.exact.max_free)
+                opt = self.exact.optimal_moves(torch.where(exact.unsqueeze(1), roots, full).contiguous(), self.exact_policy)
+                exact_seen |= exact
+                exact_rows += exact.sum()
             k = n_moves - move_i  # legal moves left: one edge is played per move
-            reads = torch.where(active, torch.full((n,), _n_searches(k, num_read), dtype=torch.int32, device=dev),
+            searched = active if exact is None else active & ~exact
+            reads = torch.where(searched, torch.full((n,), _n_searches(k, num_read), dtype=torch.int32, device=dev),
                                 torch.full((n,), -1, dtype=torch.int32, device=dev))
             noise = noise_all[move_i] * valid if noise_all is not None else None
             eng.run_search(reads, self.ev, noise=noise, coeff=coeff, max_reads=_n_searches(k, num_read), graph_waves=self.graph_waves,
                            pending=self.pending, adaptive=self.adaptive)
             vis = eng.root_visits()
             stats, _rw, q = eng.tree_stats()
+            if exact is not None:
+                vis = torch.where(exact.unsqueeze(1), opt.int(), vis)
+                stats = torch.where(exact.unsqueeze(1), torch.zeros_like(stats), stats)
+                q = torch.where(exact, torch.zeros_like(q), q)
             v = vis.double()
             probs = (v / v.max(1, keepdim=True).values.clamp_min(1.0)) ** (1.0 / temperature)
             probs = torch.where(active.unsqueeze(1), probs, valid.double())  # finished games: any legal filler, ignored below
@@ -322,6 +390,8 @@ class BatchedSelfPlay:
         info = eng.status()  # the only host synchronisation of the whole batch of games
         self.total_sims = info["sims"]
         info["adjudicated"] = int((margin != -128).sum())
+        info["exact_games"] = int(exact_seen.sum())
+        info["exact_rows"] = int(exact_rows)
         self._device_hist = dict(states=hist_states, visits=hist_visits, active=hist_active, moves=hist_moves, stats=hist_stats,
                                  q=hist_q, final=final, result=res, margin=margin, games_idxs=games_idxs, with_features=with_features,
                                  noise=noise_all)  # the pre-drawn Dirichlet samples [move, game, A]: a run can be replayed
@@ -375,6 +445,7 @@ class BatchedSelfPlay:
         moves = torch.full((n,), -1, dtype=torch.int32, device=dev)
         left_dev = torch.zeros((1,), dtype=torch.int32, device=dev)
         margin = torch.full((n,), -128, dtype=torch.int8, device=dev)  # final margin of an adjudicated game's root, else ILLEGAL
+        exact_margin = torch.full((n,), -128, dtype=torch.int8, device=dev)  # ... of the root a game was played out from, else ILLEGAL
         u_all = torch.rand((n_moves, n), dtype=torch.float64, device=dev, generator=gen)  # one uniform per (move, game): the draw of the move
 
         eng.pending = 1
@@ -394,23 +465,28 @@ class BatchedSelfPlay:
                                h_states=ptr(h_states), h_visits=ptr(h_visits), h_active=ptr(h_active), h_moves=ptr(h_moves),
                                h_stats=ptr(h_stats), h_q=ptr(h_q), noise_buf=ptr(noise_buf), reads=ptr(reads), left=ptr(left_dev))
         keep = (bufs, inv_temp, reads_by_k, u_all, noise_all)  # the kernels hold raw pointers: these tensors live until the loop ends
-        adj = self.endgame
+        adj, ex = self.endgame, self.exact
 
         eng.selfplay_restart(bufs, first=True)  # every tree begins its first search ...
         if adj is not None:
             adj.adjudicate(bufs, margin, first=True)  # ... unless its start state is adjudicated already
+        if ex is not None:
+            ex.play_out(bufs, exact_margin, self.exact_policy, first=True)  # ... or is played out exactly already
         eng.begin(reads, noise_arg, coeff, 1)
 
         def finish():
             """Trees whose search has finished: record the sample, draw the move (k_selfplay_pick), re-root
             (k_advance_roots), budget and noise of the next search (k_selfplay_restart), end the games whose new root is
-            adjudicated (k_selfplay_adjudicate, with adjudication on), begin the other searches (k_search_begin).
-            Four or five launches on in-place state, captured as one CUDA graph."""
+            adjudicated (k_selfplay_adjudicate, with adjudication on) or play them out exactly (k_selfplay_exact_endgame,
+            with exact_endgame on), begin the other searches (k_search_begin).  Four or five launches on in-place state,
+            captured as one CUDA graph."""
             eng.selfplay_pick(bufs)
             eng.advance_roots(moves, reuse=bool(sp.reuse_mcts_tree))
             eng.selfplay_restart(bufs)
             if adj is not None:
                 adj.adjudicate(bufs, margin)
+            if ex is not None:
+                ex.play_out(bufs, exact_margin, self.exact_policy)
             eng.begin(reads, noise_arg, coeff, 1)
 
         # capture_begin / capture_end directly: the torch.cuda.graph() context empties the caching allocator (and the pinned
@@ -460,10 +536,15 @@ class BatchedSelfPlay:
         info = eng.status()
         self.total_sims = info["sims"]
         info["adjudicated"] = int((margin != -128).sum())
+        info["exact_games"] = int((exact_margin != -128).sum())
+        info["exact_rows"] = 0
+        if ex is not None:  # rows of positions with f <= max_free: every one of them was played out exactly
+            rows = h_states.reshape(-1, 4)[h_active.reshape(-1)].contiguous()
+            info["exact_rows"] = int((eng.valid_moves(rows).sum(1) <= ex.max_free).sum()) if rows.shape[0] else 0
         info["checks"] = i  # finish-graph replays of the batch
         self._device_hist = dict(states=list(h_states.unbind(0)), visits=list(h_visits.unbind(0)), active=list(h_active.unbind(0)),
                                  moves=list(h_moves.unbind(0)), stats=list(h_stats.unbind(0)), q=list(h_q.unbind(0)), final=final,
-                                 result=res, margin=margin, games_idxs=games_idxs, with_features=with_features,
+                                 result=res, margin=margin, exact_margin=exact_margin, games_idxs=games_idxs, with_features=with_features,
                                  noise=noise_all if alpha > 0 else None,  # pre-drawn Dirichlet samples [move, game, A]
                                  uniforms=u_all, inv_temp=inv_temp)              # ... and what drew the moves
         del keep
@@ -486,7 +567,7 @@ class BatchedSelfPlay:
         pi = v / v.sum(1, keepdim=True).clamp_min(1.0)
         slot, mi = idx % n, idx // n
         to_play = sel.view(torch.uint8).reshape(-1, 32)[:, 20].to(torch.int8)
-        winner, outcome = _game_outcomes(h["final"], h["result"], h["margin"])
+        winner, outcome = _hist_outcomes(h)
         z_final = outcome.float()[slot]
         z = torch.where(to_play == winner[slot], z_final, -z_final)
         return planes, pi, z, slot, mi
@@ -526,7 +607,7 @@ class BatchedSelfPlay:
         move = pick(prev).astype(np.int16)
         g_of = torch.arange(n, device=act.device).unsqueeze(1).expand(n, M).reshape(-1)[sel].cpu().numpy()
         m_of = torch.arange(M, device=act.device).unsqueeze(0).expand(n, M).reshape(-1)[sel].cpu().numpy()
-        winner, res = (x.cpu().numpy() for x in _game_outcomes(h["final"], h["result"], h["margin"]))
+        winner, res = (x.cpu().numpy() for x in _hist_outcomes(h))
         res = res.astype(np.int64)
         z = np.where(player == winner[g_of], res[g_of], -res[g_of])
         games = np.asarray(h["games_idxs"])
@@ -555,7 +636,7 @@ class BatchedSelfPlay:
         """Turn the device-resident history of play_games_device() into the row dicts of get_datasets()."""
         h, eng = self._device_hist, self.eng
         n = eng.n_games
-        winner, res = (x.cpu().numpy() for x in _game_outcomes(h["final"], h["result"], h["margin"]))
+        winner, res = (x.cpu().numpy() for x in _hist_outcomes(h))
         act = torch.stack(h["active"]).cpu().numpy()
         moves = torch.stack(h["moves"]).cpu().numpy()
         vis = torch.stack(h["visits"]).cpu().numpy()

@@ -194,6 +194,17 @@ int dbaz_selfplay_restart(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, int
  * margin[t] of every other tree is not written (initialise it to -128).  Capturable in a CUDA graph. */
 int dbaz_selfplay_adjudicate(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, int8_t *margin, int32_t max_free,
                              int32_t first, uint64_t stream);
+/* Optional instead of dbaz_selfplay_adjudicate, at the same place and with the same trees: exact play.  A tree that
+ * restarted with searching[t] == 1 and whose root has at most max_free (0 .. 16) free real edges is played out from there
+ * to the first state with a result, with optimal moves (kind 0: outcome-optimal, 1: margin-optimal) and no search.  Ply j
+ * writes history row move_idx[t] + j as dbaz_selfplay_pick writes a searched root: h_states = the state, h_visits = 1 on the
+ * optimal moves and 0 elsewhere, h_stats and h_q = 0, h_moves = the move drawn from uniforms[move_idx[t] + j][t] with the
+ * weights 1, h_active = 1.  Then exact_margin[t] = the root's final margin (int8, seen by its player to move),
+ * move_idx[t] = the last row written, searching[t] = 0, reads[t] = -3 and *left is decremented.  The tree's nodes are not
+ * touched (its root stays the exact root); exact_margin[t] of every other tree is not written (initialise it to -128).
+ * Capturable in a CUDA graph. */
+int dbaz_selfplay_exact_endgame(dbaz_engine *e, const dbaz_selfplay_buffers *bufs, int8_t *exact_margin, int32_t max_free,
+                                int32_t kind, int32_t first, uint64_t stream);
 /* Synchronises `stream`.  out int64[8] = {trees with an error flag, total sims, total path nodes,
  * largest node-pool use of any tree (now or at a re-root), terminal leaves, eval-cache hits, 0, 0} (since reset_roots).  Returns non-zero (and sets
  * last_error) if any tree faulted. */
