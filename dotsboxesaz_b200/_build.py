@@ -8,8 +8,8 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "libdbaz_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["dbaz_capi.cu", "dbaz_tower.cu"]
-HEADERS = ["dbaz_device.cuh", "dbaz_game_kernels.cuh", "dbaz_tree_kernels.cuh", "dbaz_nn_kernels.cuh", "dbaz_tower.cuh", "dbaz_loop.cuh", "dbaz_selfplay.cuh", "dbaz_solver.cuh", "dbaz_endgame.cuh"]
+SOURCES = ["dbaz_capi.cu", "dbaz_tower.cu", "dbaz_trunk.cu"]
+HEADERS = ["dbaz_device.cuh", "dbaz_game_kernels.cuh", "dbaz_tree_kernels.cuh", "dbaz_nn_kernels.cuh", "dbaz_tower.cuh", "dbaz_tcgen05.cuh", "dbaz_trunk.cuh", "dbaz_loop.cuh", "dbaz_selfplay.cuh", "dbaz_solver.cuh", "dbaz_endgame.cuh"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ARCH + ["-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-I" + INCLUDE]
 

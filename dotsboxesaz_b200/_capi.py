@@ -84,6 +84,10 @@ SYMBOLS = {
     "dbaz_nn_tower_planarize": (C.c_int, [_P, _P, _P, _I64, _U64]),
     "dbaz_nn_tower": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _P, _I64, _U64]),
     "dbaz_nn_tower_trace": (C.c_int, [_P, _P]),
+    "dbaz_nn_trunk_conv_taps": (C.c_int, [_I32, _I32, _I32, _P]),
+    "dbaz_nn_trunk_conv_plan_bytes": (C.c_int64, []),
+    "dbaz_nn_trunk_conv_plan": (C.c_int, [_P, _P, _P, _P, _P, _P, _I64, _I32, _I32, _I32, _P]),
+    "dbaz_nn_trunk_conv": (C.c_int, [_P, _P, _I64, _U64]),
     "dbaz_fake_nn": (C.c_int, [_P, _P, _P, _P, _I32, _I64, _U64]),
     "dbaz_solver_solve": (C.c_int, [_P, _P, _I64, _U64]),
     "dbaz_solver_moves": (C.c_int, [_P, _P, _P, _P, _P, _I64, _U64]),
@@ -92,6 +96,7 @@ SYMBOLS = {
     "dbaz_endgame_eval": (C.c_int, [_P, _P, _P, _P, _I32, _I32, _I32, _I64, _U64]),
     "dbaz_endgame_deep_moves": (C.c_int, [_P, _P, _I64, _I32, _P, _I64, _P, _P, _U64]),
 }
+TRUNK_MAX_POS = 64  # input positions of dbaz_nn_trunk_conv (the largest board the engine plays)
 ENDGAME_DEEP_GEOM_BYTES = 512  # workspace bytes of one position's geometry in dbaz_endgame_deep_moves, beside its 2^f table
 
 _lib = None

@@ -14,6 +14,7 @@
 #include "dbaz_tree_kernels.cuh"
 #include "dbaz_selfplay.cuh"
 #include "dbaz_tower.cuh"
+#include "dbaz_trunk.cuh"
 #include "dbaz_loop.cuh"
 #include "dbaz_solver.cuh"
 #include "dbaz_endgame.cuh"
@@ -37,6 +38,7 @@ struct dbaz_engine {
     unsigned long long* d_status;
     int* d_tower_err;     // set by k_resnet_tower when a barrier wait times out
     long long* tower_dbg; // caller-owned timeline buffer (dbaz_nn_tower_trace), may be null
+    int* d_trunk_err;     // set by k_trunk_conv when a barrier wait times out
     int solver_edges;     // real edges of the board (E)
     SolverGeom sg;        // compact geometry of the exact solver, valid when solver_edges <= SOLVER_MAX_EDGES
     uint16_t* eg_order;   // endgame_order_host: the masks of every f <= 16 by popcount (ENDGAME_ORDER_ENTRIES)
@@ -328,6 +330,7 @@ void dbaz_engine_destroy(dbaz_engine* e) {
     cudaFree(e->ta.cache);
     cudaFree(e->d_status);
     cudaFree(e->d_tower_err);
+    cudaFree(e->d_trunk_err);
     cudaFree(e->d_cache_epoch);
     cudaFree(e->eg_order);
     delete e;
@@ -532,6 +535,51 @@ int dbaz_nn_tower_trace(dbaz_engine* e, int64_t* timeline) {
     if (!e) return 1;
     e->tower_dbg = reinterpret_cast<long long*>(timeline);
     return 0;
+}
+
+/* ---------------------------------------------------------- trunk convolution */
+
+int dbaz_nn_trunk_conv_taps(int32_t hi, int32_t wi, int32_t pad, int32_t* out) {
+    if (!out) return 1;
+    TrunkTaps t;
+    if (!trunk_taps(hi, wi, pad, &t).empty()) return 1;
+    out[0] = t.ho; out[1] = t.wo;
+    for (int p = 0; p < TRUNK_MAX_POS; ++p) {
+        int32_t* row = out + 2 + 10 * p;
+        row[0] = p < t.n_out ? t.count[p] : 0;
+        for (int k = 0; k < 9; ++k) row[1 + k] = (p < t.n_out && k < t.count[p]) ? (int32_t)(((t.tap[p][k] >> 4) << 8) | (t.tap[p][k] & 15)) : -1;
+        out[2 + 10 * TRUNK_MAX_POS + p] = p < t.n_out ? t.order[p] : -1;
+    }
+    return 0;
+}
+
+int64_t dbaz_nn_trunk_conv_plan_bytes(void) { return (int64_t)sizeof(TrunkPlan); }
+
+int dbaz_nn_trunk_conv_plan(dbaz_engine* e, const void* x, void* y, const void* packed_w, const float* bias_pos, const float* bias, int64_t cap,
+                            int32_t hi, int32_t wi, int32_t pad, void* plan) {
+    if (!e || !plan) return 1;
+    DeviceGuard guard(e->cfg.device);
+    if (!e->d_trunk_err) {
+        DBAZ_CK(e, cudaMalloc(&e->d_trunk_err, sizeof(int)));
+        DBAZ_CK(e, cudaMemset(e->d_trunk_err, 0, sizeof(int)));
+    }
+    TrunkPlanArgs a;
+    a.x = x; a.y = y; a.packed_w = packed_w; a.bias_pos = bias_pos; a.bias = bias; a.cap = cap; a.hi = hi; a.wi = wi; a.pad = pad;
+    a.n_sms = e->n_sms; a.err = e->d_trunk_err;
+    TrunkPlan p;
+    const std::string err = trunk_plan(a, &p);
+    if (!err.empty()) return fail(e, err);
+    memcpy(plan, &p, sizeof(p));
+    return 0;
+}
+
+int dbaz_nn_trunk_conv(dbaz_engine* e, const void* plan, int64_t n, uint64_t stream) {
+    if (!e || !plan) return 1;
+    DeviceGuard guard(e->cfg.device);
+    TrunkPlan p;  // the caller's copy need not be 64-byte aligned
+    memcpy(&p, plan, sizeof(p));
+    const std::string err = trunk_launch(p, n, S(stream));
+    return err.empty() ? 0 : fail(e, err);
 }
 
 /* ---------------------------------------------------------------- search */

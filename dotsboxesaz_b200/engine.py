@@ -24,6 +24,32 @@ class EngineError(RuntimeError):
     pass
 
 
+class TrunkConvPlan:
+    """A trunk convolution bound to its buffers (Engine.nn_trunk_conv_plan): the host bytes the launch passes to the
+    kernel, and the tensors they point to, kept alive with the plan."""
+
+    def __init__(self, buf, tensors):
+        self.buf = buf
+        self.x, self.y, self.w, self.bias_pos, self.bias = tensors
+
+
+def trunk_conv_taps(hi, wi, pad):
+    """Tap table of the trunk convolution kernel (include/dbaz_b200.h: dbaz_nn_trunk_conv_taps); needs no device.
+    Returns (ho, wo, taps, order): taps[p] = [(input position, 3 ky + kx), ...] in accumulation order, order = the output
+    positions as the kernel hands them out."""
+    out = (C.c_int32 * (2 + 11 * _capi.TRUNK_MAX_POS))()
+    if _capi.load().dbaz_nn_trunk_conv_taps(int(hi), int(wi), int(pad), out) != 0:
+        raise ValueError("trunk conv: unsupported grid %dx%d with padding %d" % (hi, wi, pad))
+    v = list(out)
+    ho, wo = v[0], v[1]
+    taps = []
+    for p in range(ho * wo):
+        row = v[2 + 10 * p: 12 + 10 * p]
+        taps.append([(e >> 8, e & 255) for e in row[1:1 + row[0]]])
+    base = 2 + 10 * _capi.TRUNK_MAX_POS
+    return ho, wo, taps, v[base: base + ho * wo]
+
+
 class Engine:
     """One engine = one GPU's shard of concurrent games (`n_games` trees of at most `max_nodes` nodes).
 
@@ -399,6 +425,30 @@ class Engine:
         self._ck(self.lib.dbaz_nn_tower(self._h, _ptr(tiles), _ptr(packed_w), _ptr(bias), int(n_stages), int(head_cout), _ptr(out), n,
                                         self._stream()))
         return out
+
+    # ------------------------------------------- SimpleNN trunk convolution (tcgen05)
+    def nn_trunk_conv_plan(self, x, y, packed_w, bias_pos, bias, pad):
+        """Binds one 256-channel 3x3 convolution (zero padding `pad`) to its buffers for nn_trunk_conv (include/dbaz_b200.h:
+        dbaz_nn_trunk_conv_plan).  x: [cap, hi, wi, 256] bf16 NHWC; y: [cap, ho, wo, 256] bf16; packed_w: trunk_conv_pack(w);
+        bias_pos: [ho * wo, 256] and bias: [256] float32, added in that order.  Encodes the tensor maps once: build plans
+        outside any stream capture."""
+        cap, hi, wi, c = x.shape
+        ho, wo = hi + 2 * pad - 2, wi + 2 * pad - 2
+        ok = (c == 256 and x.dtype == y.dtype == packed_w.dtype == torch.bfloat16 and bias_pos.dtype == bias.dtype == torch.float32
+              and tuple(y.shape) == (cap, ho, wo, 256) and tuple(packed_w.shape) == (9 * 256, 256) and tuple(bias_pos.shape) == (ho * wo, 256)
+              and tuple(bias.shape) == (256,) and all(t.is_contiguous() and t.device == self.device for t in (x, y, packed_w, bias_pos, bias)))
+        if not ok:
+            raise ValueError("nn_trunk_conv_plan: expected contiguous bf16 x [cap, hi, wi, 256], y [cap, ho, wo, 256], "
+                             "w [2304, 256] and float32 biases [ho * wo, 256], [256] on %s" % self.device)
+        buf = C.create_string_buffer(int(self.lib.dbaz_nn_trunk_conv_plan_bytes()))
+        self._ck(self.lib.dbaz_nn_trunk_conv_plan(self._h, _ptr(x), _ptr(y), _ptr(packed_w), _ptr(bias_pos), _ptr(bias), cap, hi, wi,
+                                                  int(pad), buf), launches=0)
+        return TrunkConvPlan(buf, (x, y, packed_w, bias_pos, bias))
+
+    def nn_trunk_conv(self, plan, n):
+        """Runs a planned trunk convolution for boards 0 .. n-1; returns y[:n] (rows n .. cap-1 of y are not written)."""
+        self._ck(self.lib.dbaz_nn_trunk_conv(self._h, plan.buf, int(n), self._stream()))
+        return plan.y[:n]
 
     # -------------------------------------------------------------- search
     def reset_roots(self, states=None):

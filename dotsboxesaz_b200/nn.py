@@ -433,6 +433,35 @@ def tower_reference(x_nhwc, w3, b3, w_head=None, b_head=None):
     return out.permute(0, 2, 3, 1).contiguous().to(torch.bfloat16)
 
 
+def trunk_conv_pack(w):
+    """[256 cout, 256 cin, 3, 3] weights -> the [ky][kx][cout][cin] bf16 order of Engine.nn_trunk_conv_plan, as [2304, 256]."""
+    assert tuple(w.shape) == (256, 256, 3, 3)
+    return w.permute(2, 3, 0, 1).reshape(9 * 256, 256).to(torch.bfloat16).contiguous()
+
+
+def trunk_conv_bias(bias, bpos, pad):
+    """The two biases of the trunk kernel as the library plan rounds them: the per-position map bpos [cout, ho, wo] (the
+    image of the previous BatchNorm's shift; different at each border position of a padded layer) and the conv's bias
+    [cout], each rounded to bf16 like the `z` operand and bias of cuDNN's conv-add-bias-ReLU.  pad 0: the map is one
+    constant, folded into the bias as the library plan does.  Returns (bias_pos [ho * wo, cout], bias [cout]) float32."""
+    r = lambda t: t.to(torch.bfloat16).float()
+    cout = bpos.shape[0]
+    if pad == 0:
+        return torch.zeros((bpos.shape[1] * bpos.shape[2], cout), device=bpos.device), r(bias.float() + bpos[:, 0, 0].float()).contiguous()
+    return r(bpos.float().permute(1, 2, 0).reshape(-1, cout)).contiguous(), r(bias.float()).contiguous()
+
+
+def trunk_conv_reference(x_nhwc, w, bias_pos, bias, pad):
+    """What the trunk kernel computes, in float64 on bf16-rounded weights and inputs: relu(conv(x, w) + bias_pos + bias),
+    rounded once to bf16.  x_nhwc [n, hi, wi, 256]; w [256, 256, 3, 3]; bias_pos [ho * wo, 256]; bias [256]; returns
+    [n, ho, wo, 256] bf16."""
+    r = lambda t: t.to(torch.bfloat16).double()
+    y = F.conv2d(r(x_nhwc).permute(0, 3, 1, 2), r(w), None, padding=pad)
+    n, c, ho, wo = y.shape
+    y = y + bias_pos.double().t().reshape(1, c, ho, wo) + bias.double().view(1, c, 1, 1)
+    return F.relu(y).permute(0, 2, 3, 1).to(torch.bfloat16).contiguous()
+
+
 def _copy_plan_tensors(dst, src, path="plan"):
     """dst <- src for every tensor reachable through tuples / lists / dicts of the two plans, IN PLACE (same addresses:
     CUDA graphs captured around the plan stay valid).  Structures must match; None on the src side (buffers a
@@ -473,16 +502,23 @@ class FusedSimpleNN(_ReloadablePlan):
     Every layer is conv/linear -> ReLU -> eval-mode BatchNorm (y = s*r + t).  The affine is pushed into the NEXT
     layer: its weights take the factor s per input channel and its bias takes the image of t -- a constant vector for
     the unpadded conv4 and the linear layers, a per-position map for the zero-padded 3x3 convs (the border sees fewer
-    taps), which is added as the `z` operand of cuDNN's fused conv-add-bias-ReLU.  So each layer is ONE library
-    kernel on the tensor cores with its bias/ReLU in the epilogue: cuDNN conv-(add-)bias-ReLU for the trunk,
-    cuBLASLt GEMM-bias-ReLU for the FC layers; conv0 (leaf gather + conv + ReLU straight from the packed leaf states)
-    and the softmax/tanh heads are the engine's own kernels.  fc0's columns are permuted to the NHWC flatten order,
-    policy and value heads are one GEMM.  Same function as the module in eval mode up to rounding of the compute
-    dtype (tests/test_gpu_nn.py)."""
+    taps).  So each layer is ONE kernel on the tensor cores with its bias/ReLU in the epilogue.  In bf16 at batches of
+    TRUNK_MIN_ROWS and more, the padded convs conv1-conv3 run as the engine's trunk kernel, which skips the taps that fall
+    into the padding and otherwise computes what cuDNN computes (same bf16 map and bias, same order of the sums);
+    otherwise they run as cuDNN's fused conv-add-bias-ReLU with the map as its `z` operand.  conv4 is cuDNN conv-bias-ReLU, the FC layers cuBLASLt GEMM-bias-ReLU; conv0 (leaf
+    gather + conv + ReLU straight from the packed leaf states) and the softmax/tanh heads are the engine's own kernels.
+    fc0's columns are permuted to the NHWC flatten order, policy and value heads are one GEMM.  Same function as the
+    module in eval mode up to rounding of the compute dtype (tests/test_gpu_nn.py)."""
 
-    def __init__(self, model, engine, dtype=torch.bfloat16, use_stem=True, _buffers=True):
+    # Below this many leaves the padded convs stay on cuDNN even when the trunk kernel is available: a work item is 128
+    # boards at one position, so small batches leave most SMs idle and one 9-tap item (~16 us) is the kernel's floor.
+    # tools/trunk_conv_bench.py on a B200 (1000 W), conv1 kernel / cuDNN: 18.5 / 9.4 us at 256 leaves, 19.1 / 17.1 at 768,
+    # 19.4 / 23.9 at 1024, 27.8 / 31.1 at 2048, 46.6 / 58.0 at 4096.
+    TRUNK_MIN_ROWS = 1024
+
+    def __init__(self, model, engine, dtype=torch.bfloat16, use_stem=True, use_trunk=True, _buffers=True):
         self.engine, self.dtype = engine, dtype
-        self._ctor = {"use_stem": use_stem}
+        self._ctor = {"use_stem": use_stem, "use_trunk": use_trunk}
         dev = engine.device
         model = copy.deepcopy(model).to(dev).train(False)  # never move or retype the caller's (training) module
         rows, cols = engine.rows, engine.cols
@@ -499,22 +535,47 @@ class FusedSimpleNN(_ReloadablePlan):
         else:
             self.conv0 = (_cl(c0.weight.detach(), dtype), c0.bias.detach().to(dtype), tuple(c0.padding))
         self.convs = []
+        # The zero-padded convs (conv1-conv3) as the engine's tcgen05 trunk kernel (csrc/dbaz_trunk.cu) at batches of
+        # TRUNK_MIN_ROWS and more: a GEMM per output position over its in-board taps with the z map and bias of the library
+        # path, so no padding tap is multiplied and the result is the library's.  conv4 has no padding to skip and stays on cuDNN.
+        convs = [getattr(model, f"conv{i}") for i in range(1, 5)]
+        n_trunk = 0
+        if (use_trunk and dtype == torch.bfloat16 and (self.stem_mma is not None or self.stem is not None) and c0.out_channels == 256
+                and rows * cols <= 64):
+            for c in convs:
+                if (isinstance(c, nn.Sequential) or tuple(c.kernel_size) != (3, 3) or c.in_channels != 256 or c.out_channels != 256
+                        or c.groups != 1 or tuple(c.stride) != (1, 1) or tuple(c.dilation) != (1, 1) or tuple(c.padding) != (1, 1)):
+                    break
+                n_trunk += 1
+        self.trunk = [] if n_trunk else None
+        # with the kernel, the library path (and its z maps) only serves batches below TRUNK_MIN_ROWS
+        z_rows = min(cap, self.TRUNK_MIN_ROWS) if n_trunk else cap
         hw = (rows, cols)
-        for i in range(1, 5):
-            conv = getattr(model, f"conv{i}")
+        for i, conv in enumerate(convs, 1):
             s, t = _bn_affine(getattr(model, f"bn{i - 1}"))
             w32 = conv.weight.detach().float()
             pad = tuple(conv.padding)
             tmap = t.view(1, -1, 1, 1).expand(1, t.numel(), hw[0], hw[1]).contiguous()
             bpos = F.conv2d(tmap, w32, None, padding=pad)[0]  # image of the shift t under this conv, [cout, H', W']
             bias = conv.bias.detach().float()
+            if i <= n_trunk:
+                self.trunk.append((trunk_conv_pack(w32 * s.view(1, -1, 1, 1)),) + trunk_conv_bias(bias, bpos, pad[0]))
             z = None
             if pad == (0, 0):
                 bias = bias + bpos[:, 0, 0]  # no padding: the same constant at every position
             else:
-                z = bpos.to(dtype).unsqueeze(0).expand(cap, -1, -1, -1).contiguous(memory_format=torch.channels_last)
+                z = bpos.to(dtype).unsqueeze(0).expand(z_rows, -1, -1, -1).contiguous(memory_format=torch.channels_last)
             self.convs.append((_cl(w32 * s.view(1, -1, 1, 1), dtype), bias.to(dtype), z, pad))
             hw = (bpos.shape[1], bpos.shape[2])
+        self.trunk_plans = None
+        if n_trunk and _buffers:
+            # stem_out -> ping-pong NHWC buffers; the plans bind the buffers' full capacity once
+            bufs = [torch.empty((cap, rows, cols, 256), dtype=dtype, device=dev) for _ in range(2)]
+            x, self.trunk_plans = self.stem_out, []
+            for i, (w, bp, b) in enumerate(self.trunk):
+                self.trunk_plans.append(engine.nn_trunk_conv_plan(x, bufs[i % 2], w, bp, b, 1))
+                x = bufs[i % 2]
+            self.trunk_out = x
         c_out = N_CH_OUT(model)
         s, t = _bn_affine(model.bn4)
         # fc0 over the NHWC flatten of conv4's output, bn4 folded in (per channel, any position)
@@ -536,7 +597,8 @@ class FusedSimpleNN(_ReloadablePlan):
         bh = bh + wh @ t1
         wh = wh * s1.view(1, -1)
         self.wh, self.bh = wh.to(dtype).t().contiguous(), bh.to(dtype)
-        self.engine_launches = 2 if (self.stem is not None or self.stem_mma is not None) else 1  # own kernels per batch: (stem,) heads
+        # own kernels per batch: (stem,) (trunk convs at full batches,) heads
+        self.engine_launches = (2 if (self.stem is not None or self.stem_mma is not None) else 1) + (len(self.trunk) if self.trunk else 0)
         engine.set_planes(dtype, channels_last=True)
 
     @torch.no_grad()
@@ -550,7 +612,13 @@ class FusedSimpleNN(_ReloadablePlan):
         else:
             w, b, pad = self.conv0
             x = _conv_relu(eng.planes, w, b, pad)
-        for w, b, z, pad in self.convs:
+        convs = self.convs
+        if self.trunk is not None and n >= self.TRUNK_MIN_ROWS:
+            for plan in self.trunk_plans:  # stem_out -> ping-pong buffers -> trunk_out, NHWC throughout
+                eng.nn_trunk_conv(plan, n)
+            x = self.trunk_out[:n].permute(0, 3, 1, 2)
+            convs = convs[len(self.trunk_plans):]
+        for w, b, z, pad in convs:
             x = _conv_relu(x, w, b, pad) if z is None else _conv_add_relu(x, w, z[:n], b, pad)
         x = x.permute(0, 2, 3, 1).reshape(n, -1)
         for w, b in self.fcs:

@@ -329,6 +329,29 @@ int dbaz_nn_tower(dbaz_engine *e, const void *tiles, const void *packed_w, const
  * h-block h: accumulator ready, block written}); NULL switches it off. */
 int dbaz_nn_tower_trace(dbaz_engine *e, int64_t *timeline);
 
+/* ---- one 256-channel 3x3 convolution of SimpleNN's trunk as a tcgen05 GEMM per output position
+ *      (dotsboxesaz_b200/csrc/dbaz_trunk.cu) ----
+ * y[b][p][:] = relu((sum over the taps t of p inside the grid: x[b][q_t][:] . w[t] + bias_pos[p][:]) + bias[:]), bf16 in
+ * and out, fp32 accumulation and epilogue; the taps that fall into the zero padding are never loaded or multiplied.  Each
+ * output element is accumulated in one fixed order (64-channel chunks ascending, in-board taps by (ky, kx) inside a
+ * chunk), so a board's output does not depend on n or on the row it sits in; it is cuDNN's order for the same conv, so
+ * with bf16-valued biases the result equals cuDNN's conv-add-bias-ReLU with z = bias_pos.
+ *
+ * dbaz_nn_trunk_conv_taps (no engine, no device): the tap table of a 3x3 convolution with zero padding pad (0 or 1) over
+ *   an hi x wi grid (hi * wi <= 64).  out: int32[2 + 10 * 64 + 64] = {ho, wo; for output position p = y * wo + x < ho * wo:
+ *   the tap count, then (q << 8) | (3 ky + kx) for each in-board tap by ascending (ky, kx), -1 beyond; then the output
+ *   positions in the order the kernel hands them out (descending tap count), -1 beyond}.  Returns 1 on a bad shape.
+ * dbaz_nn_trunk_conv_plan: binds one layer's buffers once and writes dbaz_nn_trunk_conv_plan_bytes() bytes to the host
+ *   buffer plan -- the tensor maps over the full capacity, so dbaz_nn_trunk_conv encodes and allocates nothing (safe
+ *   inside a stream capture).  x: [cap][hi][wi][256] bf16 (NHWC); y: [cap][ho][wo][256] bf16; packed_w: [ky][kx][cout][cin]
+ *   bf16; bias_pos: [ho * wo][256] float32; bias: [256] float32.  All 16-byte aligned; the buffers must outlive the plan.
+ * dbaz_nn_trunk_conv: runs the layer for boards 0 .. n-1 (n <= cap); rows n .. cap-1 of y are not written. */
+int dbaz_nn_trunk_conv_taps(int32_t hi, int32_t wi, int32_t pad, int32_t *out);
+int64_t dbaz_nn_trunk_conv_plan_bytes(void);
+int dbaz_nn_trunk_conv_plan(dbaz_engine *e, const void *x, void *y, const void *packed_w, const float *bias_pos, const float *bias, int64_t cap,
+                            int32_t hi, int32_t wi, int32_t pad, void *plan);
+int dbaz_nn_trunk_conv(dbaz_engine *e, const void *plan, int64_t n, uint64_t stream);
+
 /* ---- test/bench utility: deterministic stand-in for the policy/value net ----
  * (SURVEY.md 8a KAT definition; kind 0 hash-seeded, kind 1 uniform prior) over leaf_states[n]. */
 int dbaz_fake_nn(dbaz_engine *e, const dbaz_state *leaf_states, float *priors, float *values, int32_t kind,
